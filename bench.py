@@ -3,7 +3,7 @@
 batch 64 per GPU, data-parallel (DDP / NCCL gradient all-reduce) on synthetic COCO-shaped batches, bf16 autocast,
 plus the per-module roofline numbers of the hand-written kernels.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0.  Keys beyond the base contract: ``e2e`` (same metric through the user-facing
@@ -108,6 +108,25 @@ def _median_ms(fn, warm, reps):
     return statistics.median(ts)
 
 
+DUMP_MAX_ELEMS = 1 << 22   # per dumped array: 16 MB of float32 at any --scale
+
+
+def dump_outputs(out_dir, loss_items, state_dict):
+    """--dump-outputs: what the timed training step hands its caller after its last step, as float32 .npy files --
+    ``loss_items`` [box, cls, dfl] and ``model_state``, every floating state_dict entry of the trained model flattened in
+    logical (NCHW) order and concatenated in state_dict order; above DUMP_MAX_ELEMS a fixed seeded sample of it.  Two
+    builds run with the same arguments see the same inputs, so their dumps compare output for output."""
+    import numpy as np
+    import torch
+
+    flat = torch.cat([v.detach().float().reshape(-1).cpu() for v in state_dict.values() if v.dtype.is_floating_point])
+    if flat.numel() > DUMP_MAX_ELEMS:
+        flat = flat[torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss_items.npy"), loss_items.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "model_state.npy"), flat.numpy())
+
+
 def _ref_kind():
     """'reference' when the unmodified reference package is importable (oracle/_ref, made by oracle/build_ref.py, or
     /root/reference in the dev container); 'port' (oracle/modules.py in the harness graph) otherwise."""
@@ -133,11 +152,11 @@ def _make_cpu_trainer(kind):
     return tr, tr.step, tr.raw
 
 
-def cpu_reference_run(steps, warmup, batch=None, budget_s=150.0):
+def cpu_reference_run(steps, warmup, batch=None, budget_s=150.0, dump_dir=None):
     """The reference's own CPU implementation of the measured path -- the UNMODIFIED ``DetectionModel`` +
     ``v8DetectionLoss`` + trainer-style SGD/EMA step (oracle/ref_step.py over oracle/_ref), fp32, all host threads --
     for exactly ``warmup`` + ``steps`` steps.  ``batch=None``: the largest per-step batch in {64,32,16,8,4,2} whose
-    (warmup+steps) steps fit ``budget_s`` according to one probe step at batch 4."""
+    (warmup+steps) steps fit ``budget_s`` according to one probe step at batch 4.  ``dump_dir``: see dump_outputs()."""
     import torch
 
     from improving_yolov8_cbam_swinblock_b200.harness import synthetic
@@ -149,7 +168,7 @@ def cpu_reference_run(steps, warmup, batch=None, budget_s=150.0):
     except (AttributeError, OSError):
         pass
     torch.set_num_threads(cores)
-    tr, step, _ = _make_cpu_trainer(kind)
+    tr, step, model = _make_cpu_trainer(kind)
     if batch is None:
         probe = synthetic.make_batch(4, IMGSZ, NC, seed=99)
         step(probe)
@@ -166,8 +185,10 @@ def cpu_reference_run(steps, warmup, batch=None, budget_s=150.0):
         step(host)
     t0 = time.perf_counter()
     for _ in range(steps):
-        step(host)
+        items = step(host)
     dt = time.perf_counter() - t0
+    if dump_dir:
+        dump_outputs(dump_dir, items, model.state_dict())
     what = ("unmodified reference DetectionModel + v8DetectionLoss (oracle/_ref = verbatim copy of the reference package), trainer-style "
             "step (oracle/ref_step.py)") if kind == "reference" else "oracle/modules.py blocks in the harness graph (reference package not available)"
     return {"value": batch * steps / dt, "unit": "img/s", "cores": cores, "kind": kind, "batch": batch, "steps": steps, "warmup": warmup,
@@ -340,6 +361,13 @@ def print_record(line):
     _record_out.flush()
 
 
+def _at_least_one(s):
+    n = int(s)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"{n}: at least one timed step")
+    return n
+
+
 def main():
     _claim_stdout()
     if os.environ.get("B200_BENCH_WATCHDOG"):  # debugging aid: dump every thread's stack and exit if the run stalls
@@ -348,7 +376,7 @@ def main():
         faulthandler.dump_traceback_later(int(os.environ["B200_BENCH_WATCHDOG"]), exit=True)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=_at_least_one, default=20)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=PER_GPU_BATCH, help="per-GPU batch (default = BASELINE config)")
@@ -360,7 +388,11 @@ def main():
     ap.add_argument("--cudnn-benchmark", type=int, default=0, help="torch.backends.cudnn.benchmark for the stock convolutions (A/B switch)")
     ap.add_argument("--scale", default=SCALE, choices=["n", "s", "m"],
                     help="width/depth variant (BASELINE configs[3]: s/m with SwinBlock [256]/[384]); default n = the headline config")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's loss items and the trained model state as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference" and args.ref_batch is None:
+        ap.error("--dump-outputs with --impl reference needs --ref-batch: the default batch is picked from a timed probe step")
     globals()["SCALE"] = args.scale
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -375,7 +407,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        cb = cpu_reference_run(args.steps, args.warmup, batch=args.ref_batch)
+        cb = cpu_reference_run(args.steps, args.warmup, batch=args.ref_batch, dump_dir=args.dump_outputs)
         rconfig = dict(config)   # what this arm actually ran: CPU, fp32, its own per-step batch
         rconfig.update(per_gpu_batch=cb["batch"], global_batch=cb["batch"], parallelism="cpu", amp="none (fp32)", memory_format="contiguous (NCHW)",
                        l2="n/a (host cores)", device=f"host CPU, {cb['cores']} threads", sample_of_workload=cb["batch"] != args.batch,
@@ -443,12 +475,18 @@ def main():
     if rank == 0:
         sampler.start()
     launches0 = _lib.launch_count()
-    ms_dev = timed(lambda i: tr.step(dev[i % 2]), args.steps)
+    last = {}
+
+    def dev_step(i):
+        last["items"] = tr.step(dev[i % 2])
+
+    ms_dev = timed(dev_step, args.steps)
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the e2e leg below trains the model further
+        dump_outputs(args.dump_outputs, last["items"], tr.raw.state_dict())
     for i in range(2):
         tr.step_from_host(host[i % 2], host[(i + 1) % 2])
-    last = {}
 
     def e2e_step(i):
         # the next pinned batch is handed over like a data loader would: its H2D copy overlaps this step's compute

@@ -5,9 +5,19 @@ The reference's own tests hold no vectors for CBAM / SwinBlock / SPPF (SURVEY D9
 outputs and autograd gradients of the unmodified reference classes on seeded inputs -- are the parity pin
 for ``oracle/blocks.py`` and, on the GPU box (where the reference is absent), for the CUDA kernels.
 Each file is a flat npz: ``x``, ``gy`` (upstream grad), ``y``, ``gx``, ``w.<state_dict key>``, ``gw.<key>``.
+
+``python -m oracle.make_golden model`` writes the model-level fixture ``tests/golden/model/detection_n_256.npz`` instead:
+one fp32 training forward + loss + backward of YOLOv8n-CBAM-Swin (``SwinBlock [128]``) at batch 2, 256^2, nc=80 on the
+seeded synthetic batch, with weights set by ``fill_seeded`` (a per-tensor rule keyed by the state_dict name, so any model
+with the same state_dict keys gets the same weights).  It stores the three loss items, a fixed sample and the per-channel
+means of the three prediction maps, a fixed sample of the flattened parameter gradients and every gradient's norm.  The
+values come from the reference's ``DetectionModel`` + ``v8DetectionLoss`` when the reference is importable and from the
+harness graph with the oracle blocks + the harness loss otherwise; ``source`` in the file says which.
 """
+import math
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
@@ -16,6 +26,92 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import ref_loader  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+MODEL_FIXTURE = os.path.join(OUT, "model", "detection_n_256.npz")
+MODEL_BATCH, MODEL_IMGSZ, MODEL_NC, MODEL_DATA_SEED = 2, 256, 80, 5
+
+
+@torch.no_grad()
+def fill_seeded(model):
+    """Every floating state_dict entry from its own generator seeded by crc32(name): running means N(0, 0.1^2), running
+    variances U[0.5, 1.5], 1-D weights (norm affines) 1 + N(0, 0.1^2), biases N(0, 0.1^2), other weights U(+-1/sqrt(fan_in)).
+    The Detect head's output biases are set as the reference's ``Detect.bias_init`` sets them (box 1.0, class
+    log(5 / nc / (640 / stride)^2)), so the loss sits where training starts; the DFL projection (fixed arange, not trained)
+    keeps its value."""
+    detect = len(model.model) - 1
+    for name, t in model.state_dict().items():
+        if not t.dtype.is_floating_point or ".dfl." in name:
+            continue
+        g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+        parts = name.split(".")
+        if parts[:2] == ["model", str(detect)] and parts[2] in ("cv2", "cv3") and parts[4:] == ["2", "bias"]:
+            v = torch.full(t.shape, 1.0 if parts[2] == "cv2" else math.log(5 / t.numel() / (640 / (8 * 2 ** int(parts[3]))) ** 2))
+        elif name.endswith("running_mean") or name.endswith("bias"):
+            v = 0.1 * torch.randn(t.shape, generator=g)
+        elif name.endswith("running_var"):
+            v = 0.5 + torch.rand(t.shape, generator=g)
+        elif t.dim() == 1:
+            v = 1 + 0.1 * torch.randn(t.shape, generator=g)
+        else:
+            v = (2 * torch.rand(t.shape, generator=g) - 1) / (t[0].numel() ** 0.5)
+        t.copy_(v)
+
+
+def model_step(model, loss_fn):
+    """fp32 train-mode forward + loss + backward on the fixture's batch -> (prediction maps, loss items, {name: grad})."""
+    from improving_yolov8_cbam_swinblock_b200.harness import synthetic
+
+    batch = synthetic.make_batch(MODEL_BATCH, MODEL_IMGSZ, MODEL_NC, seed=MODEL_DATA_SEED)
+    model.train()
+    preds = model(batch["img"].float() / 255)
+    loss, items = loss_fn(preds, batch)
+    loss.sum().backward()
+    grads = {k: p.grad.detach().clone() for k, p in model.named_parameters() if p.grad is not None}
+    return [p.detach() for p in preds], items.detach(), grads
+
+
+def _harness_model():
+    from improving_yolov8_cbam_swinblock_b200.harness import graph, loss as hl
+    from oracle import modules as om
+
+    m = graph.DetectionGraph({"CBAM": om.CBAM, "SwinBlock": om.SwinBlock, "SPPF": om.make_sppf(graph.Conv)}, "n", MODEL_NC)
+    return m, lambda preds, batch: hl.DetectionLoss(MODEL_NC, m.stride)(preds, batch, max_boxes=8)
+
+
+def _reference_model():
+    ref_loader.import_ultralytics()
+    from ultralytics.cfg import get_cfg
+    from ultralytics.nn.tasks import DetectionModel, yaml_model_load
+    from ultralytics.utils.loss import v8DetectionLoss
+
+    d = yaml_model_load(ref_loader.REF_ROOT + "/ultralytics/cfg/models/v8/yolov8n.yaml")
+    d["backbone"][7][3] = [128]
+    d["head"][3][3] = [128]
+    m = DetectionModel(d, ch=3, nc=MODEL_NC, verbose=False)
+    m.args = get_cfg()
+    return m, lambda preds, batch: v8DetectionLoss(m)(preds, batch)
+
+
+def model_fixture(samples=4096, grad_samples=16384):
+    source = "reference" if ref_loader.available() else "harness"
+    model, loss_fn = _reference_model() if source == "reference" else _harness_model()
+    fill_seeded(model)
+    preds, items, grads = model_step(model, loss_fn)
+    g = torch.Generator().manual_seed(0)
+    d = {"source": np.array(source), "items": items.numpy()}
+    for i, p in enumerate(preds):
+        idx = torch.randperm(p.numel(), generator=g)[:samples].sort().values
+        d[f"map{i}_shape"] = np.array(p.shape)
+        d[f"map{i}_idx"], d[f"map{i}_val"] = idx.numpy().astype(np.int32), p.reshape(-1)[idx].numpy()
+        d[f"map{i}_chmean"] = p.mean((0, 2, 3)).numpy()
+    flat = torch.cat([v.reshape(-1) for v in grads.values()])
+    idx = torch.randperm(flat.numel(), generator=g)[:grad_samples].sort().values
+    d["gnames"] = np.array(list(grads))
+    d["g_idx"], d["g_val"] = idx.numpy().astype(np.int32), flat[idx].numpy()
+    d["g_norm"] = np.array([float(v.norm()) for v in grads.values()], np.float32)
+    d["gmax"] = np.array(float(flat.abs().max()), np.float32)
+    os.makedirs(os.path.dirname(MODEL_FIXTURE), exist_ok=True)
+    np.savez_compressed(MODEL_FIXTURE, **d)
+    print(f"wrote {MODEL_FIXTURE} (source: {source}, {os.path.getsize(MODEL_FIXTURE) // 1024} KiB)")
 
 
 def _run(mod, x, seed):
@@ -142,4 +238,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    model_fixture() if sys.argv[1:] == ["model"] else main()

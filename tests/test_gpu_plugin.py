@@ -12,7 +12,8 @@ import torch
 from oracle import ref_loader, ref_step
 from util import rel_err
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="oracle/_ref (reference copy) not present")]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(),
+                                                  reason="drives the reference Ultralytics package, which the repository does not ship")]
 
 
 @pytest.fixture()
