@@ -1,6 +1,5 @@
 // C-ABI plumbing: version, thread-local error string, launch accounting, device queries.
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include <atomic>
 
@@ -27,14 +26,6 @@ int check_launch(const char* what) {
     return B200_ERR_LAUNCH;
   }
   return B200_OK;
-}
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("B200_PDL");   // opt-in: measured on B200, a CUDA-graph-replayed chain gains nothing from it (profiles/README.md)
-    return e && e[0] == '1';
-  }();
-  return on;
 }
 
 int sm_count() {

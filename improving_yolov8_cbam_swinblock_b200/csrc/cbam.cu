@@ -37,7 +37,6 @@ using namespace cbam;
 // ---- pool: per-channel sum / max (+ first argmax pixel when IDX) over the CTA's pixel slice ---------------------
 template <typename T, int VW, bool IDX>
 __global__ void __launch_bounds__(kT) cbam_pool_kernel(const T* __restrict__ x, float* __restrict__ part, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float red[];   // [groups][3][C]
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nw = G.nch, groups = G.groups;
   const int p0 = s * G.np, npix = min(G.np, G.HW - p0);
@@ -99,7 +98,6 @@ __global__ void __launch_bounds__(kT) cbam_pool_kernel(const T* __restrict__ x, 
 __global__ void __launch_bounds__(kT) cbam_mlp_kernel(const float* __restrict__ part, const float* __restrict__ w1,
                                                       const float* __restrict__ w2, float* __restrict__ ca_out,
                                                       float* __restrict__ pooled, int* __restrict__ amx, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];   // pav[C] | pmx[C] | hid[2r]
   const int b = blockIdx.x, C = G.C, r = G.r, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float* pav = sm;
@@ -143,7 +141,6 @@ __global__ void __launch_bounds__(kT) cbam_mlp_kernel(const float* __restrict__ 
 template <typename T, int VW, bool IDX>
 __global__ void __launch_bounds__(kT) cbam_map_kernel(const T* __restrict__ x, const float* __restrict__ ca,
                                                       float* __restrict__ maps, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float cas[];   // [C] when a lane owns more than one channel vector
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nch = G.nch, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int p0 = s * G.np, npix = min(G.np, G.HW - p0);
@@ -240,7 +237,6 @@ template <typename T, int VW>
 __global__ void __launch_bounds__(kT) cbam_gate_kernel(const T* __restrict__ x, const float* __restrict__ ca,
                                                        const float* __restrict__ maps, const float* __restrict__ wsa,
                                                        T* __restrict__ out, float* __restrict__ sa_out, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];   // wsas[112] | tile[2][th][tw] | sas[np] | cas[C]
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nch = G.nch, W = G.W, tw = G.tw;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -345,7 +341,6 @@ template <typename T, int VW>
 __global__ void __launch_bounds__(kT) cbam_bwd_gz_kernel(const T* __restrict__ x, const T* __restrict__ g,
                                                          const float* __restrict__ ca, const float* __restrict__ sa,
                                                          float* __restrict__ gz, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float cas[];
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nch = G.nch, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int p0 = s * G.np, npix = min(G.np, G.HW - p0);
@@ -413,7 +408,6 @@ __global__ void __launch_bounds__(kT) cbam_bwd_mid_kernel(const T* __restrict__ 
                                                           const float* __restrict__ maps, const float* __restrict__ wsa,
                                                           float4* __restrict__ pixg, float* __restrict__ cpart,
                                                           float* __restrict__ gpart, T* __restrict__ gx_sa, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];   // wsas[112] | tile[3][th][tw] | pix float4[np] | gzs[np] | poff[np] | red
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nch = G.nch, W = G.W, tw = G.tw, HW = G.HW;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -538,7 +532,6 @@ __global__ void __launch_bounds__(kT) cbam_mlp_bwd_kernel(const float* __restric
                                                           const float* __restrict__ ca, const float* __restrict__ pooled,
                                                           const float* __restrict__ w1, const float* __restrict__ w2,
                                                           float* __restrict__ part, float* __restrict__ vec, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];   // pav[C] | pmx[C] | ga[C] | hid[3r]
   const int b = blockIdx.x, C = G.C, r = G.r, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   float* pav = sm;
@@ -596,7 +589,6 @@ template <typename T, int VW>
 __global__ void __launch_bounds__(kT) cbam_bwd_fin_kernel(const T* __restrict__ g, const float* __restrict__ ca,
                                                           const float4* __restrict__ pixg, const float* __restrict__ vec,
                                                           const int* __restrict__ amx, T* __restrict__ gx, const Geo G) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];   // cas[C] | gav[C]   (when a lane owns more than one channel vector)
   const int s = blockIdx.x, b = blockIdx.y, C = G.C, nch = G.nch, HW = G.HW;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -667,7 +659,6 @@ __global__ void __launch_bounds__(kT) cbam_bwd_fin_kernel(const T* __restrict__ 
 __global__ void __launch_bounds__(256) fold_partials_kernel(const float* __restrict__ part, const float* __restrict__ cpart,
                                                             float* gw1, float* gw2, float* gwsa, int B, int BS, int n1,
                                                             int n2, int ks) {
-  pdl_enter();
   const int lane = threadIdx.x & 31;
   const int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int n = n1 + n2;
@@ -770,21 +761,21 @@ int run_fwd(const void* x, const float* w1, const float* w2, const float* wsa, v
     const size_t sm1 = (size_t)G.groups * G.C * 12;
     if (stash) {
       if (int rc = ensure_smem(cbam_pool_kernel<T, VW, true>, sm1, "cbam_fwd")) return rc;
-      launch_k(cbam_pool_kernel<T, VW, true>, grid, kT, sm1, st, xt, ws.part, G);
+      cbam_pool_kernel<T, VW, true><<<grid, kT, sm1, st>>>(xt, ws.part, G);
     } else {
       if (int rc = ensure_smem(cbam_pool_kernel<T, VW, false>, sm1, "cbam_fwd")) return rc;
-      launch_k(cbam_pool_kernel<T, VW, false>, grid, kT, sm1, st, xt, ws.part, G);
+      cbam_pool_kernel<T, VW, false><<<grid, kT, sm1, st>>>(xt, ws.part, G);
     }
-    launch_k(cbam_mlp_kernel, G.B, kT, (size_t)(2 * G.C + 2 * G.r) * 4, st, ws.part, w1, w2, ca, sh.pooled, sh.amx, G);
+    cbam_mlp_kernel<<<G.B, kT, (size_t)(2 * G.C + 2 * G.r) * 4, st>>>(ws.part, w1, w2, ca, sh.pooled, sh.amx, G);
     if (G.mode == B200_CBAM_CA) return check_launch("cbam_fwd");
   }
   const float* cap = G.mode == B200_CBAM_SA ? nullptr : ca;
   const size_t sm2 = G.one ? 0 : (size_t)G.C * 4;
-  if (stash) launch_k(cbam_map_kernel<T, VW, true>, grid, kT, sm2, st, xt, cap, sh.maps, G);
-  else launch_k(cbam_map_kernel<T, VW, false>, grid, kT, sm2, st, xt, cap, sh.maps, G);
+  if (stash) cbam_map_kernel<T, VW, true><<<grid, kT, sm2, st>>>(xt, cap, sh.maps, G);
+  else cbam_map_kernel<T, VW, false><<<grid, kT, sm2, st>>>(xt, cap, sh.maps, G);
   const size_t sm3 = (size_t)(NTAPS + 2 * G.th * G.tw + ((G.np + 3) & ~3) + (G.one ? 0 : G.C)) * 4;
   if (int rc = ensure_smem(cbam_gate_kernel<T, VW>, sm3, "cbam_fwd")) return rc;
-  launch_k(cbam_gate_kernel<T, VW>, grid, kT, sm3, st, xt, cap, sh.maps, wsa, G.mode == B200_CBAM_FULL ? (T*)out : nullptr, sa_out, G);
+  cbam_gate_kernel<T, VW><<<grid, kT, sm3, st>>>(xt, cap, sh.maps, wsa, G.mode == B200_CBAM_FULL ? (T*)out : nullptr, sa_out, G);
   return check_launch("cbam_fwd");
 }
 
@@ -801,23 +792,23 @@ int run_bwd(const void* g, const void* x, const float* w1, const float* w2, cons
   if (G.mode != B200_CBAM_CA) {
     const float* gzin = (const float*)g;   // SA mode: dL/dsa
     if (G.mode == B200_CBAM_FULL) {
-      launch_k(cbam_bwd_gz_kernel<T, VW>, grid, kT, smc, st, xt, (const T*)g, ca, sa, ws.gz, G);
+      cbam_bwd_gz_kernel<T, VW><<<grid, kT, smc, st>>>(xt, (const T*)g, ca, sa, ws.gz, G);
       gzin = ws.gz;
     }
     const size_t smm = (size_t)(NTAPS + ((3 * G.th * G.tw + 3) & ~3) + npad * 4 + npad + npad + G.groups * G.C) * 4;
     if (int rc = ensure_smem(cbam_bwd_mid_kernel<T, VW>, smm, "cbam_bwd")) return rc;
-    launch_k(cbam_bwd_mid_kernel<T, VW>, grid, kT, smm, st, xt, G.mode == B200_CBAM_FULL ? (const T*)g : nullptr, gzin, sa, sh.maps,
+    cbam_bwd_mid_kernel<T, VW><<<grid, kT, smm, st>>>(xt, G.mode == B200_CBAM_FULL ? (const T*)g : nullptr, gzin, sa, sh.maps,
                                                       wsa, G.mode == B200_CBAM_FULL ? ws.pixg : nullptr, ws.cpart, ws.gpart,
                                                       (T*)gx, G);
   }
   if (G.mode != B200_CBAM_SA) {
-    launch_k(cbam_mlp_bwd_kernel, G.B, kT, (size_t)(3 * G.C + 3 * G.r) * 4, st, ws.gpart, G.mode == B200_CBAM_CA ? (const float*)g : nullptr, ca, sh.pooled, w1, w2, ws.part, ws.vec, G);
-    launch_k(cbam_bwd_fin_kernel<T, VW>, grid, kT, 2 * smc, st, G.mode == B200_CBAM_FULL ? (const T*)g : nullptr, ca, ws.pixg, ws.vec,
+    cbam_mlp_bwd_kernel<<<G.B, kT, (size_t)(3 * G.C + 3 * G.r) * 4, st>>>(ws.gpart, G.mode == B200_CBAM_CA ? (const float*)g : nullptr, ca, sh.pooled, w1, w2, ws.part, ws.vec, G);
+    cbam_bwd_fin_kernel<T, VW><<<grid, kT, 2 * smc, st>>>(G.mode == B200_CBAM_FULL ? (const T*)g : nullptr, ca, ws.pixg, ws.vec,
                                                           sh.amx, (T*)gx, G);
   }
   const int n1 = G.mode != B200_CBAM_SA ? G.r * G.C : 0, n2 = n1;
   const int outs = n1 + n2 + (G.mode != B200_CBAM_CA ? 2 * G.ksa * G.ksa : 0);
-  launch_k(fold_partials_kernel, (outs + 7) / 8, 256, 0, st, ws.part, ws.cpart, gw1, gw2, G.mode != B200_CBAM_CA ? gwsa : nullptr, G.B,
+  fold_partials_kernel<<<(outs + 7) / 8, 256, 0, st>>>(ws.part, ws.cpart, gw1, gw2, G.mode != B200_CBAM_CA ? gwsa : nullptr, G.B,
                                                        G.B * G.S, n1, n2, G.ksa);
   return check_launch("cbam_bwd");
 }

@@ -18,7 +18,6 @@
 // owns ~50 pixels at the model's shape, so scalar set-up code is what the kernel's latency is made of.
 // With a stash the kernel also writes the by-products the (streaming) backward of cbam.cu consumes.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include <map>
 #include <mutex>
@@ -111,7 +110,6 @@ __device__ __forceinline__ void channel_partials(const T* xc, int np, int p0, in
 
 template <typename T, int VW, bool IDX>
 __global__ void __launch_bounds__(kT) cbam_cluster_fwd_kernel(const __grid_constant__ Params P) {
-  pdl_enter();
   cg::cluster_group cluster = cg::this_cluster();
   const Plan& L = P.pl;
   const int CS = L.cs, rank = blockIdx.x, b = blockIdx.y;
@@ -407,15 +405,13 @@ int launch(K kern, const Params& P, cudaStream_t st) {
   cfg.blockDim = dim3(kT);
   cfg.dynamicSmemBytes = L.total;
   cfg.stream = st;
-  cudaLaunchAttribute at[2];
+  cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = L.cs;
   at[0].val.clusterDim.y = 1;
   at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // see common.cuh: the kernel starts with pdl_enter()
-  at[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 1;
   // can this device co-schedule one such cluster at all (MIG slices, small GPCs, 16-CTA non-portable clusters)?  Asked once
   // per (kernel, cluster size, smem); 0 or a failed launch -> -1 = "not taken", the caller runs the streaming chain (cbam.cu)
   static std::mutex mu;
@@ -457,19 +453,16 @@ int cluster_fwd(const void* x, const float* w1, const float* w2, const float* ws
   L.lpp = 1;
   while (L.lpp < L.nch && L.lpp < 32) L.lpp <<= 1;
   L.groups = L.nch >= kT ? 1 : std::min(kT / L.nch, std::max(1, 13312 / (C * 12)));   // keeps 4 CTAs per SM at C=256
-  { static const int fg = [] { const char* e = getenv("B200_CBAM_GROUPS"); return e ? atoi(e) : 0; }(); if (fg > 0 && L.nch < kT) L.groups = std::min(kT / L.nch, fg); }
   L.invC = 1.f / (float)C;
   L.invHW = 1.f / (float)L.HW;
   // whole image in the shared memory of one cluster, at least two CTAs per SM so the phases of different clusters
   // overlap; bulk copies need 16-byte chunk sizes
   bool ok = false;
-  static const int forced = [] { const char* e = getenv("B200_CBAM_CS"); return e ? atoi(e) : 0; }();   // tuning aid: force the cluster size
   for (int c : {8, 16}) {
-    if (forced > 0) c = forced;
     L.cs = c; L.pchunk = (L.HW + c - 1) / c; L.cper = (C + c - 1) / c;
     if (((size_t)L.pchunk * C * esize) % 16) continue;
     layout(L, esize);
-    if ((size_t)L.total <= (size_t)(forced > 0 ? 220 : 100) * 1024) { ok = true; break; }
+    if (L.total <= 100 * 1024) { ok = true; break; }
   }
   if (!ok) return -1;
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {

@@ -25,36 +25,6 @@ int check_launch(const char* what);
 int sm_count();
 int max_smem_optin();
 
-// ---- programmatic dependent launch (PDL) ----------------------------------------------------------------------
-// A kernel launched through launch_k() carries cudaLaunchAttributeProgrammaticStreamSerialization: its CTAs may become
-// resident while the preceding kernel of the stream is still running (from the moment every CTA of that kernel has
-// executed pdl_trigger() or exited), so launch latency, CTA ramp-up and the kernel's own set-up code overlap the
-// predecessor's tail.  The contract every such kernel keeps: pdl_wait() -- which returns only when the preceding grid
-// has COMPLETED and its writes are visible -- comes before the first global-memory access (read or write).  By induction
-// over the stream order that preserves ordinary stream semantics for memory.  The edges survive stream capture
-// (programmatic dependency edges of the CUDA graph).  The attribute is OPT-IN (B200_PDL=1 in the environment): measured on
-// B200, graph-replayed kernel chains already start ~3 us apart and gain nothing from it (profiles/pdl_probe.py); without the
-// attribute pdl_wait() / pdl_trigger() are no-ops.
-bool pdl_enabled();
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_enter() { pdl_trigger(); pdl_wait(); }
-
-template <typename... P, typename... A>
-inline cudaError_t launch_k(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<P>(args)...);
-}
-
 // ---- dtype helpers ------------------------------------------------------------------------------------
 template <typename T> struct DT;
 template <> struct DT<float> {

@@ -78,7 +78,6 @@ template <typename T>
 __global__ void __launch_bounds__(kThreads, 2) conv3_dgrad_s2_kernel(const T* __restrict__ gy, const T* __restrict__ w, const WStride ws,
                                                                       T* __restrict__ gx, int H, int W, int Ho, int Wo, int tiles_per_img,
                                                                       int n_tiles) {
-  pdl_enter();
   extern __shared__ __align__(128) unsigned char smem[];
   const int RP = (Wo + 1) * kGP;                       // bytes per staged gy row
   unsigned char* gs = smem;                            // [kR + 1][Wo + 1][kGP]
@@ -201,7 +200,6 @@ template <typename T>
 __global__ void __launch_bounds__(kFThreads, 2) conv3_fwd_s2_kernel(const T* __restrict__ x, const T* __restrict__ w, const WStride ws,
                                                                      T* __restrict__ y, int H, int W, int Ho, int Wo, int tiles_per_img,
                                                                      int n_tiles) {
-  pdl_enter();
   extern __shared__ __align__(128) unsigned char smem[];
   constexpr int IR = 2 * kFR + 1;
   const int RPB = ((W + 1 + 3) / 4) * 128;             // bytes per staged input row: slot 0 = x = -1, slots 1..W, rounded up to a line
@@ -336,7 +334,7 @@ extern "C" B200_API int b200_conv3x3_dgrad_s2(const void* gy, const void* w, con
     per_sm = per_sm < 1 ? 1 : per_sm > 4 ? 4 : per_sm;
     int grid = sm_count() * per_sm;   // persistent CTAs: one resident wave
     if (grid > n_tiles) grid = n_tiles;
-    launch_k(kern, grid, kThreads, smem, st, (const T*)gy, (const T*)w, ws, (T*)gx, H, W, Ho, Wo, tpi, n_tiles);
+    kern<<<grid, kThreads, smem, st>>>((const T*)gy, (const T*)w, ws, (T*)gx, H, W, Ho, Wo, tpi, n_tiles);
     return check_launch("conv3x3_dgrad_s2");
   };
   if (dtype == B200_BF16) return go(conv3_dgrad_s2_kernel<__nv_bfloat16>, (__nv_bfloat16*)nullptr);
@@ -361,7 +359,7 @@ extern "C" B200_API int b200_conv3x3_fwd_s2(const void* x, const void* w, const 
     per_sm = per_sm < 1 ? 1 : per_sm > 4 ? 4 : per_sm;
     int grid = sm_count() * per_sm;   // persistent CTAs: one resident wave
     if (grid > n_tiles) grid = n_tiles;
-    launch_k(kern, grid, kFThreads, smem, st, (const T*)x, (const T*)w, ws, (T*)y, H, W, Ho, Wo, tpi, n_tiles);
+    kern<<<grid, kFThreads, smem, st>>>((const T*)x, (const T*)w, ws, (T*)y, H, W, Ho, Wo, tpi, n_tiles);
     return check_launch("conv3x3_fwd_s2");
   };
   if (dtype == B200_BF16) return go(conv3_fwd_s2_kernel<__nv_bfloat16>, (__nv_bfloat16*)nullptr);

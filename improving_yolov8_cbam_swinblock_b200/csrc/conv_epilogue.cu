@@ -107,7 +107,6 @@ __device__ __forceinline__ void cta_fold(float* red, int C, int ngrp, F emit) {
 template <typename T, int VW>
 __global__ void __launch_bounds__(kT, 4) bn_stats_kernel(const T* __restrict__ x, float* __restrict__ part, const BnGeo G) {
   extern __shared__ __align__(16) float red[];   // [ngrp][2][C]
-  pdl_enter();
   const int C = G.C, tpr = G.tpr;
   const int rg = threadIdx.x / tpr, ch = threadIdx.x - rg * tpr;
   const long long r0 = (long long)blockIdx.x * G.rpb;
@@ -151,7 +150,6 @@ __global__ void __launch_bounds__(kFT) bn_final_kernel(const T* __restrict__ x, 
   // kFW warps per channel: the G partial rows (up to 16 per SM) are summed by 256 lanes with 2 loads in flight each --
   // one warp per channel made this 8-CTA kernel a 10 us latency chain, 59 times per step (2982 -> 3123 img/s)
   __shared__ float fs[kFT / 32][2];
-  pdl_enter();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, sub = warp % kFW, C = G.C;
   const int c = blockIdx.x * (kFT / 32 / kFW) + warp / kFW;
   const bool live = c < C;
@@ -203,7 +201,6 @@ template <typename T, int VW, int ACT>
 __global__ void __launch_bounds__(kT, 4) bn_apply_kernel(const T* __restrict__ x, const float* __restrict__ scsh,
                                                       T* __restrict__ z, const BnGeo G) {
   constexpr bool FAST = sizeof(T) == 2;
-  pdl_enter();
   const int C = G.C, tpr = G.tpr;
   const int rg = threadIdx.x / tpr, ch = threadIdx.x - rg * tpr;
   if (rg >= G.ngrp) return;
@@ -249,7 +246,6 @@ __global__ void __launch_bounds__(kT, 4) bn_bwd_reduce_kernel(const T* __restric
                                                            float* __restrict__ part, const long long gzs, const BnGeo G) {
   constexpr bool FAST = sizeof(T) == 2;   // gzs: row stride of gz in elements (the gradient of a concat slice is a strided view)
   extern __shared__ __align__(16) float red[];   // [ngrp][2][C]
-  pdl_enter();
   const int C = G.C, tpr = G.tpr;
   const int rg = threadIdx.x / tpr, ch = threadIdx.x - rg * tpr;
   const long long r0 = (long long)blockIdx.x * G.rpb;
@@ -303,7 +299,6 @@ __global__ void __launch_bounds__(kFT) bn_bwd_final_kernel(const float* __restri
                                                           float* __restrict__ ggamma, float* __restrict__ gbeta,
                                                           float* __restrict__ coef, int training, const BnGeo G) {
   __shared__ float fs[kFT / 32][2];
-  pdl_enter();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, sub = warp % kFW, C = G.C;
   const int c = blockIdx.x * (kFT / 32 / kFW) + warp / kFW;
   const bool live = c < C;
@@ -345,7 +340,6 @@ __global__ void __launch_bounds__(kT, 4) bn_bwd_apply_kernel(const T* __restrict
                                                           const BnGeo G) {
   constexpr bool FAST = sizeof(T) == 2;
   extern __shared__ __align__(16) float cs[];   // [5][C]: a, b (y = x*a + b), A, Bc, Cc
-  pdl_enter();
   const int C = G.C, tpr = G.tpr;
   for (int c = threadIdx.x; c < C; c += kT) {
     const float a = gamma[c] * rstd[c];
@@ -475,11 +469,11 @@ extern "C" B200_API int b200_bn_silu_fwd_tracked(const void* x, const float* gam
   const size_t smem = (size_t)G.ngrp * 2 * C * 4;
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
     constexpr int VW = 16 / (int)sizeof(T);
-    if (training) launch_k(bn_stats_kernel<T, VW>, G.G, kT, smem, st, (const T*)x, part, G);
-    launch_k(bn_final_kernel<T>, (C * kFW + kFT / 32 - 1) / (kFT / 32), kFT, 0, st, (const T*)x, part, gamma, beta, running_mean, running_var,
-             mean_out, rstd_out, scsh, eps, momentum, training, (long long*)num_batches_tracked, G);
-    if (act) launch_k(bn_apply_kernel<T, VW, 1>, G.G, kT, 0, st, (const T*)x, scsh, (T*)z, G);
-    else launch_k(bn_apply_kernel<T, VW, 0>, G.G, kT, 0, st, (const T*)x, scsh, (T*)z, G);
+    if (training) bn_stats_kernel<T, VW><<<G.G, kT, smem, st>>>((const T*)x, part, G);
+    bn_final_kernel<T><<<(C * kFW + kFT / 32 - 1) / (kFT / 32), kFT, 0, st>>>((const T*)x, part, gamma, beta, running_mean, running_var,
+              mean_out, rstd_out, scsh, eps, momentum, training, (long long*)num_batches_tracked, G);
+    if (act) bn_apply_kernel<T, VW, 1><<<G.G, kT, 0, st>>>((const T*)x, scsh, (T*)z, G);
+    else bn_apply_kernel<T, VW, 0><<<G.G, kT, 0, st>>>((const T*)x, scsh, (T*)z, G);
     return check_launch("bn_silu_fwd");
   });
 }
@@ -503,12 +497,12 @@ extern "C" B200_API int b200_bn_silu_bwd(const void* gz, int64_t gz_row_stride, 
   const size_t smem = (size_t)G.ngrp * 2 * C * 4;
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
     constexpr int VW = 16 / (int)sizeof(T);
-    if (act) launch_k(bn_bwd_reduce_kernel<T, VW, 1>, G.G, kT, smem, st, (const T*)x, (const T*)gz, gamma, beta, mean, rstd, part, gzs, G);
-    else launch_k(bn_bwd_reduce_kernel<T, VW, 0>, G.G, kT, smem, st, (const T*)x, (const T*)gz, gamma, beta, mean, rstd, part, gzs, G);
-    launch_k(bn_bwd_final_kernel, (C * kFW + kFT / 32 - 1) / (kFT / 32), kFT, 0, st, part, gamma, mean, rstd, ggamma, gbeta, coef, training, G);
+    if (act) bn_bwd_reduce_kernel<T, VW, 1><<<G.G, kT, smem, st>>>((const T*)x, (const T*)gz, gamma, beta, mean, rstd, part, gzs, G);
+    else bn_bwd_reduce_kernel<T, VW, 0><<<G.G, kT, smem, st>>>((const T*)x, (const T*)gz, gamma, beta, mean, rstd, part, gzs, G);
+    bn_bwd_final_kernel<<<(C * kFW + kFT / 32 - 1) / (kFT / 32), kFT, 0, st>>>(part, gamma, mean, rstd, ggamma, gbeta, coef, training, G);
     const size_t smc = (size_t)5 * C * 4;
-    if (act) launch_k(bn_bwd_apply_kernel<T, VW, 1>, G.G, kT, smc, st, (const T*)x, (const T*)gz, gamma, beta, mean, rstd, coef, (T*)gx, gzs, G);
-    else launch_k(bn_bwd_apply_kernel<T, VW, 0>, G.G, kT, smc, st, (const T*)x, (const T*)gz, gamma, beta, mean, rstd, coef, (T*)gx, gzs, G);
+    if (act) bn_bwd_apply_kernel<T, VW, 1><<<G.G, kT, smc, st>>>((const T*)x, (const T*)gz, gamma, beta, mean, rstd, coef, (T*)gx, gzs, G);
+    else bn_bwd_apply_kernel<T, VW, 0><<<G.G, kT, smc, st>>>((const T*)x, (const T*)gz, gamma, beta, mean, rstd, coef, (T*)gx, gzs, G);
     return check_launch("bn_silu_bwd");
   });
 }

@@ -43,7 +43,6 @@ template <typename T, int OC, int S>
 __global__ void __launch_bounds__(WarpPlan<OC>::NW * 32, 2) conv3_wgrad_kernel(const T* __restrict__ gy, const T* __restrict__ x,
                                                                                 float* __restrict__ part, int H, int W, int Ho, int Wo,
                                                                                 int tiles_per_img, int n_tiles) {
-  pdl_enter();
   using WP = WarpPlan<OC>;
   constexpr int R = TileRows<S>::R, IR = TileRows<S>::IR, MT = OC / 16, NT = kCin / 8, PB = kCin * 2, NTH = WP::NW * 32, TPW = WP::TPW;
   // shared-memory pixel pitches: 16 bytes of padding per pixel, so that the eight 16-byte rows of an ldmatrix tile (consecutive pixels,
@@ -145,7 +144,6 @@ __global__ void __launch_bounds__(WarpPlan<OC>::NW * 32, 2) conv3_wgrad_kernel(c
 
 // gw[oc][c][ky][kx] = sum over CTAs of part[cta][ky * 3 + kx][oc][c]; warp per element, fixed-order butterfly
 __global__ void __launch_bounds__(256) conv3_wgrad_fold_kernel(const float* __restrict__ part, int n_part, int OC, int CIN, float* __restrict__ gw) {
-  pdl_enter();
   const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (i >= OC * CIN * 9) return;
   const int oc = i / (CIN * 9), rem = i - oc * CIN * 9, c = rem / 9, tap = rem - c * 9;
@@ -180,9 +178,9 @@ int launch_wgrad(const void* gy, const void* x, float* gw, float* part, int n_ct
   int grid = sm_count() * per_sm;
   if (grid > n_tiles) grid = n_tiles;
   if (grid > n_ctas_max) grid = n_ctas_max;
-  launch_k(kern, grid, NTH, smem, st, (const T*)gy, (const T*)x, part, H, W, Ho, Wo, tpi, n_tiles);
+  kern<<<grid, NTH, smem, st>>>((const T*)gy, (const T*)x, part, H, W, Ho, Wo, tpi, n_tiles);
   if (int rc = check_launch("conv3x3_wgrad")) return rc;
-  launch_k(conv3_wgrad_fold_kernel, (OC * kCin * 9 * 32 + 255) / 256, 256, 0, st, part, grid, OC, kCin, gw);
+  conv3_wgrad_fold_kernel<<<(OC * kCin * 9 * 32 + 255) / 256, 256, 0, st>>>(part, grid, OC, kCin, gw);
   return check_launch("conv3x3_wgrad_fold");
 }
 

@@ -192,7 +192,6 @@ __device__ __forceinline__ float align_metric(const DetParams& P, float score, f
 // ---------------------------------------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(256) det_decode_kernel(const DetParams P) {
-  pdl_enter();
   const long long gi = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long r = gi >> 2;
   const int side = (int)(gi & 3);
@@ -224,7 +223,6 @@ __global__ void __launch_bounds__(256) det_decode_kernel(const DetParams P) {
 }
 
 __global__ void __launch_bounds__(256) tal_topk_kernel(const DetParams P) {
-  pdl_enter();
   extern __shared__ float sm[];
   float* s_align = sm;                 // [A_total]
   float* s_ovl = sm + P.A_total;       // [A_total]
@@ -289,7 +287,6 @@ __global__ void __launch_bounds__(256) tal_topk_kernel(const DetParams P) {
 }
 
 __global__ void __launch_bounds__(256) tal_resolve_kernel(const DetParams P) {
-  pdl_enter();
   extern __shared__ int s_sel[];   // [nmax * topk] selected anchors of this image
   const int b = blockIdx.y, n = P.nmax * P.topk;
   for (int e = threadIdx.x; e < n; e += blockDim.x) s_sel[e] = P.sel_idx[(size_t)b * n + e];
@@ -329,7 +326,6 @@ __global__ void __launch_bounds__(256) tal_resolve_kernel(const DetParams P) {
 }
 
 __global__ void __launch_bounds__(256) tal_finish_kernel(const DetParams P) {
-  pdl_enter();
   const int b = blockIdx.y;
   const int a = blockIdx.x * blockDim.x + threadIdx.x;
   if (a >= P.A_total) return;
@@ -394,7 +390,6 @@ __device__ __forceinline__ void dfl_target(float dist, int* tl, float* wl) {
 
 template <typename T>
 __global__ void __launch_bounds__(256) box_dfl_fwd_kernel(const DetParams P) {
-  pdl_enter();
   float acc_box = 0.f, acc_dfl = 0.f;
   for (long long r0 = (long long)blockIdx.x * blockDim.x + threadIdx.x; r0 < P.rows_total; r0 += (long long)gridDim.x * blockDim.x) {
     long long r = r0;
@@ -439,7 +434,6 @@ __global__ void __launch_bounds__(256) box_dfl_fwd_kernel(const DetParams P) {
   }
 }
 __global__ void __launch_bounds__(256) fold2_kernel(const float* __restrict__ part, int n, float* __restrict__ out) {
-  pdl_enter();
   __shared__ float red[8][2];
   float s0 = 0.f, s1 = 0.f;
   for (int i = threadIdx.x; i < n; i += 256) { s0 += part[2 * i]; s1 += part[2 * i + 1]; }
@@ -456,7 +450,6 @@ __global__ void __launch_bounds__(256) fold2_kernel(const float* __restrict__ pa
 
 template <typename T>
 __global__ void __launch_bounds__(256) box_dfl_bwd_kernel(const DetParams P) {
-  pdl_enter();
   const float g_box = P.gscale[0], g_dfl = P.gscale[1];
   const long long gi = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long r = gi >> 2;
@@ -537,9 +530,9 @@ extern "C" B200_API int b200_det_decode(const void* const* box_maps, const void*
   const long long threads = P.rows_total * 4;
   const int grid = (int)((threads + 255) / 256);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B200_F32) launch_k(det_decode_kernel<float>, grid, 256, 0, st, P);
-  else if (dtype == B200_BF16) launch_k(det_decode_kernel<__nv_bfloat16>, grid, 256, 0, st, P);
-  else launch_k(det_decode_kernel<__half>, grid, 256, 0, st, P);
+  if (dtype == B200_F32) det_decode_kernel<float><<<grid, 256, 0, st>>>(P);
+  else if (dtype == B200_BF16) det_decode_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(P);
+  else det_decode_kernel<__half><<<grid, 256, 0, st>>>(P);
   return check_launch("det_decode");
 }
 
@@ -574,14 +567,14 @@ extern "C" B200_API int b200_tal_assign(const float* pred_boxes, const float* sc
   const size_t smem_topk = (size_t)P.A_total * 8;
   B200_REQUIRE(smem_topk <= (size_t)max_smem_optin(), B200_ERR_UNSUPPORTED, "tal_assign: %d anchors do not fit in shared memory", P.A_total);
   cudaFuncSetAttribute(tal_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_topk);
-  launch_k(tal_topk_kernel, B * nmax, 256, smem_topk, st, P);
+  tal_topk_kernel<<<B * nmax, 256, smem_topk, st>>>(P);
   if (int rc = check_launch("tal_topk")) return rc;
   const dim3 grid((P.A_total + 255) / 256, B);
   const size_t smem_sel = (size_t)nmax * topk * 4;
   B200_REQUIRE(smem_sel <= 48 * 1024, B200_ERR_UNSUPPORTED, "tal_assign: nmax * topk = %d too large", nmax * topk);
-  launch_k(tal_resolve_kernel, grid, 256, smem_sel, st, P);
+  tal_resolve_kernel<<<grid, 256, smem_sel, st>>>(P);
   if (int rc = check_launch("tal_resolve")) return rc;
-  launch_k(tal_finish_kernel, grid, 256, 0, st, P);
+  tal_finish_kernel<<<grid, 256, 0, st>>>(P);
   return check_launch("tal_finish");
 }
 
@@ -599,11 +592,11 @@ extern "C" B200_API int b200_box_dfl_fwd(const void* const* box_maps, const int3
   P.tbox = const_cast<float*>(target_box); P.tvalue = const_cast<float*>(weight); P.part = (float*)workspace;
   const int grid = sm_count() * 4;
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B200_F32) launch_k(box_dfl_fwd_kernel<float>, grid, 256, 0, st, P);
-  else if (dtype == B200_BF16) launch_k(box_dfl_fwd_kernel<__nv_bfloat16>, grid, 256, 0, st, P);
-  else launch_k(box_dfl_fwd_kernel<__half>, grid, 256, 0, st, P);
+  if (dtype == B200_F32) box_dfl_fwd_kernel<float><<<grid, 256, 0, st>>>(P);
+  else if (dtype == B200_BF16) box_dfl_fwd_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(P);
+  else box_dfl_fwd_kernel<__half><<<grid, 256, 0, st>>>(P);
   if (int rc = check_launch("box_dfl_fwd")) return rc;
-  launch_k(fold2_kernel, 1, 256, 0, st, P.part, grid, sums);
+  fold2_kernel<<<1, 256, 0, st>>>(P.part, grid, sums);
   return check_launch("box_dfl_fold");
 }
 
@@ -619,8 +612,8 @@ extern "C" B200_API int b200_box_dfl_bwd(const void* const* box_maps, void* cons
   const long long threads = P.rows_total * 4;
   const int grid = (int)((threads + 255) / 256);
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B200_F32) launch_k(box_dfl_bwd_kernel<float>, grid, 256, 0, st, P);
-  else if (dtype == B200_BF16) launch_k(box_dfl_bwd_kernel<__nv_bfloat16>, grid, 256, 0, st, P);
-  else launch_k(box_dfl_bwd_kernel<__half>, grid, 256, 0, st, P);
+  if (dtype == B200_F32) box_dfl_bwd_kernel<float><<<grid, 256, 0, st>>>(P);
+  else if (dtype == B200_BF16) box_dfl_bwd_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(P);
+  else box_dfl_bwd_kernel<__half><<<grid, 256, 0, st>>>(P);
   return check_launch("box_dfl_bwd");
 }

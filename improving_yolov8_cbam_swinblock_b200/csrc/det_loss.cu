@@ -35,7 +35,6 @@ __device__ __forceinline__ float softplus_f(float x) { return fmaxf(x, 0.f) + __
 
 template <typename T, int VE, bool BWD>
 __global__ void __launch_bounds__(256) bce_kernel(const BceParams P) {
-  pdl_enter();
   const int vpr = P.C / VE;   // vectors per row
   float acc = 0.f;
   const float sc = BWD ? P.scale[0] : 0.f;
@@ -100,7 +99,6 @@ __global__ void __launch_bounds__(256) bce_kernel(const BceParams P) {
 }
 
 __global__ void __launch_bounds__(256) bce_fold_kernel(const float* __restrict__ part, int n, float* __restrict__ out) {
-  pdl_enter();
   __shared__ float red[8];
   float s = 0.f;
   for (int i = threadIdx.x; i < n; i += 256) s += part[i];
@@ -151,11 +149,11 @@ extern "C" B200_API int b200_bce_logits_fwd(const void* const* logits, const int
   const int grid = sm_count() * 8;
   P.part = (float*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B200_F32) launch_k(bce_kernel<float, 4, false>, grid, 256, 0, st, P);
-  else if (dtype == B200_BF16) launch_k(bce_kernel<__nv_bfloat16, 8, false>, grid, 256, 0, st, P);
-  else launch_k(bce_kernel<__half, 8, false>, grid, 256, 0, st, P);
+  if (dtype == B200_F32) bce_kernel<float, 4, false><<<grid, 256, 0, st>>>(P);
+  else if (dtype == B200_BF16) bce_kernel<__nv_bfloat16, 8, false><<<grid, 256, 0, st>>>(P);
+  else bce_kernel<__half, 8, false><<<grid, 256, 0, st>>>(P);
   if (int rc = check_launch("bce_logits_fwd")) return rc;
-  launch_k(bce_fold_kernel, 1, 256, 0, st, P.part, grid, loss_sum);
+  bce_fold_kernel<<<1, 256, 0, st>>>(P.part, grid, loss_sum);
   return check_launch("bce_logits_fold");
 }
 
@@ -168,8 +166,8 @@ extern "C" B200_API int b200_bce_logits_bwd(const void* const* logits, void* con
   P.scale = scale;
   const int grid = sm_count() * 8;
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == B200_F32) launch_k(bce_kernel<float, 4, true>, grid, 256, 0, st, P);
-  else if (dtype == B200_BF16) launch_k(bce_kernel<__nv_bfloat16, 8, true>, grid, 256, 0, st, P);
-  else launch_k(bce_kernel<__half, 8, true>, grid, 256, 0, st, P);
+  if (dtype == B200_F32) bce_kernel<float, 4, true><<<grid, 256, 0, st>>>(P);
+  else if (dtype == B200_BF16) bce_kernel<__nv_bfloat16, 8, true><<<grid, 256, 0, st>>>(P);
+  else bce_kernel<__half, 8, true><<<grid, 256, 0, st>>>(P);
   return check_launch("bce_logits_bwd");
 }

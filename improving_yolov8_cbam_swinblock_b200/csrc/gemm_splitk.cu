@@ -27,7 +27,6 @@ struct SplitParams {
 template <int A_MN, int B_MN>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, SplitParams P) {
-  pdl_enter();
   extern __shared__ unsigned char smem_raw_[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw_) + 1023) & ~(uintptr_t)1023);
   unsigned char* sA = smem;
@@ -157,7 +156,6 @@ gemm_splitk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 // out[i] = sum over splits (fixed order); the last `ncs` entries of every split go to `colsum`
 __global__ void fold_splits_kernel(const float* __restrict__ part, float* __restrict__ out, float* __restrict__ colsum, int splits,
                                    size_t n, size_t ncs) {
-  pdl_enter();
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n + ncs) return;
   float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
@@ -223,12 +221,12 @@ extern "C" B200_API int b200_gemm_splitk(const void* A, const void* B, float* D,
   {                                                                                               \
     auto k = gemm_splitk_kernel<AM, BMN>;                                                         \
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL);             \
-    launch_k(k, grid, kThreads, SMEM_TOTAL, st, *mA, *mB, P);                                           \
+    k<<<grid, kThreads, SMEM_TOTAL, st>>>(*mA, *mB, P);                                           \
   }
   if (a_mn && b_mn) LAUNCH_SK(1, 1) else if (a_mn) LAUNCH_SK(1, 0) else if (b_mn) LAUNCH_SK(0, 1) else LAUNCH_SK(0, 0)
 #undef LAUNCH_SK
   if (int rc = check_launch("gemm_splitk")) return rc;
   const size_t n = (size_t)M * N;
-  launch_k(fold_splits_kernel, (unsigned)((n + M + 255) / 256), 256, 0, st, (const float*)workspace, D, colsum, splits, n, (size_t)M);
+  fold_splits_kernel<<<(unsigned)((n + M + 255) / 256), 256, 0, st>>>((const float*)workspace, D, colsum, splits, n, (size_t)M);
   return check_launch("gemm_splitk_fold");
 }

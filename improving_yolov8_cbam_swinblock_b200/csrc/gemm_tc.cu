@@ -186,7 +186,6 @@ __global__ void __launch_bounds__(Thr<EW>::kThreads, 1)
 gemm_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmD, const __grid_constant__ CUtensorMap tmD2,
                const __grid_constant__ CUtensorMap tmR, GemmParams P) {
-  pdl_enter();
   using S = Smem<BLOCK_N, STAGES, NBUF, (EPI == EPI_BIAS ? 0 : NBUF)>;
   constexpr int kEpiThreads = Thr<EW>::kEpiThreads;
   extern __shared__ unsigned char smem_raw_[];
@@ -410,7 +409,7 @@ int launch(const void* A, const void* B, const float* bias, void* D, void* D2, c
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL);
   int grid = P.m_tiles * P.n_tiles;
   if (grid > sm_count()) grid = sm_count();
-  launch_k(kern, grid, Thr<EW>::kThreads, S::TOTAL, st, *mA, *mB, *mD, *mD2, *mR, P);
+  kern<<<grid, Thr<EW>::kThreads, S::TOTAL, st>>>(*mA, *mB, *mD, *mD2, *mR, P);
   return check_launch("gemm_nt");
 }
 

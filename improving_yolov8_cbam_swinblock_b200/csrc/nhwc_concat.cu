@@ -43,7 +43,6 @@ struct CatParams {
 
 template <typename V>   // V = uint4 (16-byte vectors) or a 2/4-byte scalar
 __global__ void __launch_bounds__(kT) nhwc_concat_kernel(const __grid_constant__ CatParams P) {
-  pdl_enter();
   const uint32_t step = gridDim.x * kT;
   for (uint32_t i0 = blockIdx.x * kT + threadIdx.x; i0 < P.items; i0 += kInFlight * step) {
     V v[kInFlight];
@@ -109,9 +108,9 @@ extern "C" B200_API int b200_nhwc_concat(const void* const* srcs, const int32_t*
   const long long cap = (long long)sm_count() * 16;
   if (blocks > cap) blocks = cap;
   cudaStream_t st = (cudaStream_t)stream;
-  if (vec) launch_k(nhwc_concat_kernel<uint4>, (unsigned)blocks, kT, 0, st, P);
-  else if (es == 4) launch_k(nhwc_concat_kernel<uint32_t>, (unsigned)blocks, kT, 0, st, P);
-  else launch_k(nhwc_concat_kernel<uint16_t>, (unsigned)blocks, kT, 0, st, P);
+  if (vec) nhwc_concat_kernel<uint4><<<(unsigned)blocks, kT, 0, st>>>(P);
+  else if (es == 4) nhwc_concat_kernel<uint32_t><<<(unsigned)blocks, kT, 0, st>>>(P);
+  else nhwc_concat_kernel<uint16_t><<<(unsigned)blocks, kT, 0, st>>>(P);
   return check_launch("nhwc_concat");
 }
 
@@ -173,7 +172,6 @@ template <typename T> __device__ __forceinline__ uint4 add_pack(const float* v) 
 
 template <typename T, int N>
 __global__ void __launch_bounds__(kT) nhwc_add_kernel(const __grid_constant__ AddParams P) {
-  pdl_enter();
   constexpr int VW = 16 / (int)sizeof(T);
   constexpr int U = N <= 2 ? 4 : 2;   // vectors in flight per thread and source
   const uint32_t step = gridDim.x * kT;
@@ -240,9 +238,9 @@ extern "C" B200_API int b200_nhwc_add(const void* const* srcs, const int64_t* sr
   if (blocks > cap) blocks = cap;
   cudaStream_t st = (cudaStream_t)stream;
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
-    if (n_src == 2) launch_k(nhwc_add_kernel<T, 2>, (unsigned)blocks, kT, 0, st, P);
-    else if (n_src == 3) launch_k(nhwc_add_kernel<T, 3>, (unsigned)blocks, kT, 0, st, P);
-    else launch_k(nhwc_add_kernel<T, 4>, (unsigned)blocks, kT, 0, st, P);
+    if (n_src == 2) nhwc_add_kernel<T, 2><<<(unsigned)blocks, kT, 0, st>>>(P);
+    else if (n_src == 3) nhwc_add_kernel<T, 3><<<(unsigned)blocks, kT, 0, st>>>(P);
+    else nhwc_add_kernel<T, 4><<<(unsigned)blocks, kT, 0, st>>>(P);
     return check_launch("nhwc_add");
   });
 }
@@ -260,7 +258,6 @@ namespace {
 template <typename T, int CH>
 __global__ void __launch_bounds__(256) u8_to_nhwc_kernel(const uint8_t* __restrict__ img, T* __restrict__ out, long long hw,
                                                          long long quads, float inv) {
-  pdl_enter();
   // thread = 4 consecutive pixels of one image: CH uchar4 loads (one per plane), 4*CH contiguous output elements
   for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < quads; q += (long long)gridDim.x * blockDim.x) {
     const long long hq = hw / 4;
@@ -293,10 +290,10 @@ int launch_u8(const uint8_t* img, void* out, int B, int C, long long hw, float i
   const long long cap = (long long)sm_count() * 32;
   if (blocks > cap) blocks = cap;
   switch (C) {
-    case 1: launch_k(u8_to_nhwc_kernel<T, 1>, (unsigned)blocks, 256, 0, st, img, (T*)out, hw, quads, inv); break;
-    case 2: launch_k(u8_to_nhwc_kernel<T, 2>, (unsigned)blocks, 256, 0, st, img, (T*)out, hw, quads, inv); break;
-    case 3: launch_k(u8_to_nhwc_kernel<T, 3>, (unsigned)blocks, 256, 0, st, img, (T*)out, hw, quads, inv); break;
-    default: launch_k(u8_to_nhwc_kernel<T, 4>, (unsigned)blocks, 256, 0, st, img, (T*)out, hw, quads, inv); break;
+    case 1: u8_to_nhwc_kernel<T, 1><<<(unsigned)blocks, 256, 0, st>>>(img, (T*)out, hw, quads, inv); break;
+    case 2: u8_to_nhwc_kernel<T, 2><<<(unsigned)blocks, 256, 0, st>>>(img, (T*)out, hw, quads, inv); break;
+    case 3: u8_to_nhwc_kernel<T, 3><<<(unsigned)blocks, 256, 0, st>>>(img, (T*)out, hw, quads, inv); break;
+    default: u8_to_nhwc_kernel<T, 4><<<(unsigned)blocks, 256, 0, st>>>(img, (T*)out, hw, quads, inv); break;
   }
   return check_launch("u8_to_nhwc");
 }
@@ -333,7 +330,6 @@ struct UpGeo {
 };
 
 __global__ void __launch_bounds__(256) upsample_fwd_kernel(const uint4* __restrict__ x, uint4* __restrict__ out, const __grid_constant__ UpGeo G) {
-  pdl_enter();
   const uint32_t step = gridDim.x * 256;
   for (uint32_t i = blockIdx.x * 256 + threadIdx.x; i < G.items; i += step) {
     const uint32_t pix = G.dvpp.div(i), v = i - pix * G.vpp;
@@ -347,7 +343,6 @@ __global__ void __launch_bounds__(256) upsample_fwd_kernel(const uint4* __restri
 template <typename T>
 __global__ void __launch_bounds__(256) upsample_bwd_kernel(const unsigned char* __restrict__ g, uint4* __restrict__ gin,
                                                            const __grid_constant__ UpGeo G) {
-  pdl_enter();
   constexpr int VW = 16 / (int)sizeof(T);
   const uint32_t step = gridDim.x * 256;
   for (uint32_t i = blockIdx.x * 256 + threadIdx.x; i < G.items; i += step) {
@@ -402,7 +397,7 @@ extern "C" B200_API int b200_nhwc_upsample_fwd(const void* x, void* out, int32_t
   B200_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 15) == 0, B200_ERR_ALIGN, "nhwc_upsample_fwd: tensors must be 16-byte aligned");
   UpGeo G;
   if (int rc = up_geo(G, B, C, H, W, sh, sw, dtype, false, 0)) return rc;
-  launch_k(upsample_fwd_kernel, up_blocks(G.items), 256, 0, (cudaStream_t)stream, static_cast<const uint4*>(x), static_cast<uint4*>(out), G);
+  upsample_fwd_kernel<<<up_blocks(G.items), 256, 0, (cudaStream_t)stream>>>(static_cast<const uint4*>(x), static_cast<uint4*>(out), G);
   return check_launch("nhwc_upsample_fwd");
 }
 
@@ -414,7 +409,7 @@ extern "C" B200_API int b200_nhwc_upsample_bwd(const void* gout, int64_t gout_ro
   if (int rc = up_geo(G, B, C, H, W, sh, sw, dtype, true, gout_row_stride)) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
-    launch_k(upsample_bwd_kernel<T>, up_blocks(G.items), 256, 0, st, static_cast<const unsigned char*>(gout), static_cast<uint4*>(gin), G);
+    upsample_bwd_kernel<T><<<up_blocks(G.items), 256, 0, st>>>(static_cast<const unsigned char*>(gout), static_cast<uint4*>(gin), G);
     return check_launch("nhwc_upsample_bwd");
   });
 }

@@ -12,8 +12,6 @@
 // Backward: the per-stage winners (row offset, col offset: 4+4 bits) are recomputed from y0 with the same rule,
 // then gradients are routed stage 3 -> 1 by two 1-D scatters per stage.  Every strip (row / column, channel)
 // is owned by exactly one thread, so the scatter is race-free and summation order is fixed: deterministic.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "sppf_word.cuh"
 
@@ -276,7 +274,6 @@ struct PoolGeom {
 template <typename T, int K, int LP, bool WITH_IDX>
 __global__ void __launch_bounds__(512) sppf_pool_fwd_kernel(const T* __restrict__ y0, T* __restrict__ cat,
                                                             int32_t* __restrict__ idx, PoolGeom g) {
-  pdl_enter();
   using WD = Word<T>;
   constexpr int EPL = WD::EPL;
   constexpr int CC = LP * EPL;
@@ -397,7 +394,6 @@ __device__ __forceinline__ void scatter1d(const float* __restrict__ src, int sst
 template <typename T, int K, int LP>
 __global__ void __launch_bounds__(512) sppf_pool_bwd_kernel(const T* __restrict__ gcat, const T* __restrict__ y0,
                                                             T* __restrict__ gy0, PoolGeom g) {
-  pdl_enter();
   using WD = Word<T>;
   constexpr int EPL = WD::EPL;
   constexpr int CC = LP * EPL;
@@ -560,7 +556,6 @@ __device__ __forceinline__ void ring_walk(Ring<K>& rg, float* buf, int stride, c
 template <typename T, int K, int LP, int MAXT>   // MAXT 320: registers capped for 4 (K <= 5) / 3 CTAs per SM
 __global__ void __launch_bounds__(MAXT, MAXT <= 320 ? (K <= 5 ? 4 : 3) : 1) sppf_pool_bwd_inplace_kernel(const T* __restrict__ gcat, const T* __restrict__ y0,
                                                                     T* __restrict__ gy0, PoolGeom g) {
-  pdl_enter();
   using WD = Word<T>;
   constexpr int EPL = WD::EPL;
   static_assert(EPL == 2, "in-place variant: 16-bit dtypes");
@@ -663,11 +658,11 @@ int launch_fwd(const void* y0, void* cat, int32_t* idx, PoolGeom g, cudaStream_t
   if (idx) {
     auto kern = sppf_pool_fwd_kernel<T, K, LP, true>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_k(kern, grid, threads, smem, st, (const T*)y0, (T*)cat, idx, g);
+    kern<<<grid, threads, smem, st>>>((const T*)y0, (T*)cat, idx, g);
   } else {
     auto kern = sppf_pool_fwd_kernel<T, K, LP, false>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_k(kern, grid, threads, smem, st, (const T*)y0, (T*)cat, idx, g);
+    kern<<<grid, threads, smem, st>>>((const T*)y0, (T*)cat, idx, g);
   }
   return check_launch("sppf_pool_fwd");
 }
@@ -685,16 +680,14 @@ int launch_bwd(const void* gcat, const void* y0, void* gy0, PoolGeom g, cudaStre
   // two segments per strip measured best (89 us vs 107 with one, 97 with three at 64x128x20x20): the kernel is bound by
   // instruction issue, and every extra segment re-scans K-1 sources
   while (g.nseg < 2 && strips * (g.nseg + 1) * LP <= 512 && (g.H < g.W ? g.H : g.W) / (g.nseg + 1) >= K) ++g.nseg;
-  if (const char* ov = getenv("B200_SPPF_NSEG")) g.nseg = atoi(ov) > 0 ? atoi(ov) : g.nseg;   // tuning aid
   if constexpr (EPL == 2) {
     // 16-bit dtypes, two segments per strip, every strip covered in one sweep: in-place routing (one gradient buffer)
     const int per = ((strips * LP + 31) / 32) * 32;
-    const char* off = getenv("B200_SPPF_NO_INPLACE");
-    if (g.nseg == 2 && 2 * per <= 512 && g.H >= 2 && g.W >= 2 && !(off && off[0] == '1')) {
+    if (g.nseg == 2 && 2 * per <= 512 && g.H >= 2 && g.W >= 2) {
       const size_t smem_ip = plane * LP * EPL * 4 + plane * LP * 6;
       auto kip = 2 * per <= 320 ? sppf_pool_bwd_inplace_kernel<T, K, LP, 320> : sppf_pool_bwd_inplace_kernel<T, K, LP, 512>;
       cudaFuncSetAttribute(kip, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ip);
-      launch_k(kip, dim3(g.B * chunks), 2 * per, smem_ip, st, (const T*)gcat, (const T*)y0, (T*)gy0, g);
+      kip<<<dim3(g.B * chunks), 2 * per, smem_ip, st>>>((const T*)gcat, (const T*)y0, (T*)gy0, g);
       return check_launch("sppf_pool_bwd");
     }
   }
@@ -703,7 +696,7 @@ int launch_bwd(const void* gcat, const void* y0, void* gy0, PoolGeom g, cudaStre
   if (threads < 64) threads = 64;
   auto kern = sppf_pool_bwd_kernel<T, K, LP>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  launch_k(kern, dim3(g.B * chunks), threads, smem, st, (const T*)gcat, (const T*)y0, (T*)gy0, g);
+  kern<<<dim3(g.B * chunks), threads, smem, st>>>((const T*)gcat, (const T*)y0, (T*)gy0, g);
   return check_launch("sppf_pool_bwd");
 }
 

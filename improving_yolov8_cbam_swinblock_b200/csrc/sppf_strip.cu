@@ -131,7 +131,6 @@ __device__ __forceinline__ void strip_route(SRC src, OFF off, DST dst) {
 template <typename T, int K>
 __global__ void __launch_bounds__(NT, 2) sppf_strip_bwd_kernel(const T* __restrict__ gcat, const T* __restrict__ y0, T* __restrict__ gy0,
                                                                int C) {
-  pdl_enter();
   using WD = Word<T>;
   using PR = Pair<T>;
   extern __shared__ __align__(16) uint32_t smem[];
@@ -240,7 +239,6 @@ __global__ void __launch_bounds__(NT, 2) sppf_strip_bwd_kernel(const T* __restri
 
 template <typename T, int K>
 __global__ void __launch_bounds__(NT, 3) sppf_strip_fwd_kernel(const T* __restrict__ y0, T* __restrict__ cat, int C) {
-  pdl_enter();
   using WD = Word<T>;
   extern __shared__ __align__(16) uint32_t smem[];
   uint32_t* Bp = smem;
@@ -313,7 +311,7 @@ int launch_bwd(const void* gcat, const void* y0, void* gy0, int B, int C, cudaSt
   constexpr int smem = PW * 8 + PW * 6;
   auto kern = sppf_strip_bwd_kernel<T, K>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  launch_k(kern, B * (C / (2 * CW)), NT, smem, st, (const T*)gcat, (const T*)y0, (T*)gy0, C);
+  kern<<<B * (C / (2 * CW)), NT, smem, st>>>((const T*)gcat, (const T*)y0, (T*)gy0, C);
   return check_launch("sppf_pool_bwd(strip)");
 }
 template <typename T, int K>
@@ -321,7 +319,7 @@ int launch_fwd(const void* y0, void* cat, int B, int C, cudaStream_t st) {
   constexpr int smem = PW * 8;
   auto kern = sppf_strip_fwd_kernel<T, K>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  launch_k(kern, B * (C / (2 * CW)), NT, smem, st, (const T*)y0, (T*)cat, C);
+  kern<<<B * (C / (2 * CW)), NT, smem, st>>>((const T*)y0, (T*)cat, C);
   return check_launch("sppf_pool_fwd(strip)");
 }
 

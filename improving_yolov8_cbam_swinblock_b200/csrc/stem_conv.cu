@@ -83,7 +83,6 @@ __device__ __forceinline__ void stage_input(unsigned char* xs, const T* __restri
 template <typename T, int OC>
 __global__ void __launch_bounds__(256) stem_fwd_kernel(const T* __restrict__ x, const float* __restrict__ w, T* __restrict__ y, int H, int W,
                                                        int Ho, int Wo, int tiles_per_img, int pitch) {
-  pdl_enter();
   extern __shared__ __align__(16) unsigned char xs[];
   constexpr int NT = OC / 8;
   const int b = blockIdx.x / tiles_per_img, oy0 = (blockIdx.x - b * tiles_per_img) * kR;
@@ -136,7 +135,6 @@ __global__ void __launch_bounds__(256) stem_fwd_kernel(const T* __restrict__ x, 
 template <typename T, int OC>
 __global__ void __launch_bounds__(256) stem_wgrad_kernel(const T* __restrict__ gy, const T* __restrict__ x, float* __restrict__ part, int H,
                                                          int W, int Ho, int Wo, int tiles_per_img, int n_tiles, int pitch) {
-  pdl_enter();
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr int MT = OC / 16;
   unsigned char* xs = smem;                                  // 2 * kRW + 1 input rows
@@ -211,7 +209,6 @@ __global__ void __launch_bounds__(256) stem_wgrad_kernel(const T* __restrict__ g
 // dW[oc][c][ky][kx] = sum over CTAs of part[cta][oc][10 * ky + 1 + 3 * kx + c]: one warp per element, lanes stride over the CTAs
 // (independent loads; one thread walking all partials was a 100 us chain of L2 latencies), fixed-order butterfly: deterministic
 __global__ void __launch_bounds__(256) stem_wgrad_fold_kernel(const float* __restrict__ part, int n_part, int OC, float* __restrict__ gw) {
-  pdl_enter();
   const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (i >= OC * 27) return;
   const int oc = i / 27, rem = i - oc * 27, c = rem / 9, ky = (rem - c * 9) / 3, kx = rem - c * 9 - ky * 3;
@@ -254,7 +251,7 @@ extern "C" B200_API int b200_stem_conv_fwd(const void* x, const float* w, void* 
   {                                                                                                            \
     auto kern = stem_fwd_kernel<TT, OCC>;                                                                      \
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                        \
-    launch_k(kern, B * tpi, 256, smem, st, (const TT*)x, w, (TT*)y, H, W, Ho, Wo, tpi, pitch);                       \
+    kern<<<B * tpi, 256, smem, st>>>((const TT*)x, w, (TT*)y, H, W, Ho, Wo, tpi, pitch);                       \
   }
   if (dtype == B200_BF16) {
     if (c2 == 16) B200_STEM_FWD(__nv_bfloat16, 16) else if (c2 == 32) B200_STEM_FWD(__nv_bfloat16, 32) else B200_STEM_FWD(__nv_bfloat16, 48)
@@ -288,7 +285,7 @@ extern "C" B200_API int b200_stem_conv_wgrad(const void* gy, const void* x, floa
     per_sm = per_sm < 1 ? 1 : per_sm > 5 ? 5 : per_sm;                                                         \
     grid = sm_count() * per_sm;                                                                                \
     if (grid > n_tiles) grid = n_tiles;                                                                        \
-    launch_k(kern, grid, 256, smem, st, (const TT*)gy, (const TT*)x, part, H, W, Ho, Wo, tpi, n_tiles, pitch);       \
+    kern<<<grid, 256, smem, st>>>((const TT*)gy, (const TT*)x, part, H, W, Ho, Wo, tpi, n_tiles, pitch);       \
   }
   if (dtype == B200_BF16) {
     if (c2 == 16) B200_STEM_WG(__nv_bfloat16, 16) else if (c2 == 32) B200_STEM_WG(__nv_bfloat16, 32) else B200_STEM_WG(__nv_bfloat16, 48)
@@ -297,6 +294,6 @@ extern "C" B200_API int b200_stem_conv_wgrad(const void* gy, const void* x, floa
   }
 #undef B200_STEM_WG
   if (int rc = check_launch("stem_conv_wgrad")) return rc;
-  launch_k(stem_wgrad_fold_kernel, (c2 * 27 * 32 + 255) / 256, 256, 0, st, part, grid, c2, gw);
+  stem_wgrad_fold_kernel<<<(c2 * 27 * 32 + 255) / 256, 256, 0, st>>>(part, grid, c2, gw);
   return check_launch("stem_conv_wgrad_fold");
 }

@@ -23,7 +23,6 @@ template <typename T> __device__ __forceinline__ float ldf(const T* p) { return 
 template <typename T>
 __global__ void __launch_bounds__(LMAX) swin_attn_fwd_kernel(const T* __restrict__ qkv, T* __restrict__ o, float* __restrict__ lse,
                                                              int L, int C, int nh, const ShiftMask M) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];
   const int hd = C / nh, hp = hd + 4;
   float* ks = sm;             // [L][hp]
@@ -87,7 +86,6 @@ template <typename T>
 __global__ void __launch_bounds__(LMAX) swin_attn_bwd_kernel(const T* __restrict__ qkv, const T* __restrict__ o,
                                                              const float* __restrict__ lse, const T* __restrict__ go,
                                                              T* __restrict__ gqkv, int L, int C, int nh, const ShiftMask M) {
-  pdl_enter();
   extern __shared__ __align__(16) float sm[];
   const int hd = C / nh, hp = hd + 4, lp = L + 1;
   float* b0 = sm;               // phase 1: K rows     phase 2: dO rows
@@ -211,7 +209,7 @@ extern "C" B200_API int b200_swin_attn_fwd(const void* qkv, void* o, float* lse,
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
     auto k = swin_attn_fwd_kernel<T>;
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_k(k, grid, LMAX, smem, (cudaStream_t)stream, (const T*)qkv, (T*)o, lse, L, C, nh, M);
+    k<<<grid, LMAX, smem, (cudaStream_t)stream>>>((const T*)qkv, (T*)o, lse, L, C, nh, M);
     return check_launch("swin_attn_fwd");
   });
 }
@@ -230,7 +228,7 @@ extern "C" B200_API int b200_swin_attn_bwd(const void* qkv, const void* o, const
   return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
     auto k = swin_attn_bwd_kernel<T>;
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_k(k, grid, LMAX, smem, (cudaStream_t)stream, (const T*)qkv, (const T*)o, lse, (const T*)go, (T*)gqkv, L, C, nh, M);
+    k<<<grid, LMAX, smem, (cudaStream_t)stream>>>((const T*)qkv, (const T*)o, lse, (const T*)go, (T*)gqkv, L, C, nh, M);
     return check_launch("swin_attn_bwd");
   });
 }

@@ -88,7 +88,6 @@ swin_attn_block_fwd_kernel(const __grid_constant__ CUtensorMap tmX, const __grid
                            const __grid_constant__ CUtensorMap tmWin, const __grid_constant__ CUtensorMap tmWo,
                            const __grid_constant__ CUtensorMap tmN1, const __grid_constant__ CUtensorMap tmQKV,
                            const __grid_constant__ CUtensorMap tmO, ABParams P) {
-  pdl_enter();
   using S = ABSmem;
   extern __shared__ __align__(1024) unsigned char smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
@@ -554,6 +553,6 @@ extern "C" B200_API int b200_swin_attn_block_fwd(const void* x, const float* gam
   const int grid = P.n_tiles < sm_count() ? P.n_tiles : sm_count();
   auto kern = dtype == B200_BF16 ? swin_attn_block_fwd_kernel<1> : swin_attn_block_fwd_kernel<0>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ABSmem::TOTAL);
-  launch_k(kern, grid, kThreads, ABSmem::TOTAL, (cudaStream_t)stream, *mX, *mY, *mWi, *mWo, *mN1, *mQ, *mO, P);
+  kern<<<grid, kThreads, ABSmem::TOTAL, (cudaStream_t)stream>>>(*mX, *mY, *mWi, *mWo, *mN1, *mQ, *mO, P);
   return check_launch("swin_attn_block_fwd");
 }

@@ -50,7 +50,6 @@ __device__ __forceinline__ uint32_t pack2f(float lo, float hi, int fmt) {
 
 template <int HD>
 __global__ void __launch_bounds__(kThreads10, 1) swin_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmO, AttnParams P) {
-  pdl_enter();
   using Cfg = ACfg<HD>;
   constexpr int KB = Cfg::KB, STAGES = Cfg::STAGES;
   extern __shared__ unsigned char smem_raw_[];
@@ -314,7 +313,7 @@ int launch_fwd(const void* qkv, void* o, float* lse, long long T, int L, int C, 
   auto k = swin_attn_fwd_tc_kernel<HD>;
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::TOTAL);
   int grid = P.n_pairs < sm_count() ? P.n_pairs : sm_count();
-  launch_k(k, grid, kThreads10, Cfg::TOTAL, st, *m, *mo, P);
+  k<<<grid, kThreads10, Cfg::TOTAL, st>>>(*m, *mo, P);
   return check_launch("swin_attn_fwd_tc");
 }
 
@@ -366,7 +365,6 @@ template <int HD>
 __global__ void __launch_bounds__(kThreads10, 1)
 swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmGO,
                         const __grid_constant__ CUtensorMap tmOut, AttnBwdParams P) {
-  pdl_enter();
   using Cfg = BCfg<HD>;
   constexpr int KB = Cfg::KB, STAGES = Cfg::STAGES, KBS = Cfg::KB_STRIDE;
   extern __shared__ unsigned char smem_raw_[];
@@ -713,7 +711,7 @@ int launch_bwd(const void* qkv, const float* lse, const void* go, void* gqkv, lo
   auto k = swin_attn_bwd_tc_kernel<HD>;
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::TOTAL);
   int grid = P.n_pairs < sm_count() ? P.n_pairs : sm_count();
-  launch_k(k, grid, kThreads10, Cfg::TOTAL, st, *m, *mg, *mo, P);
+  k<<<grid, kThreads10, Cfg::TOTAL, st>>>(*m, *mg, *mo, P);
   return check_launch("swin_attn_bwd_tc");
 }
 

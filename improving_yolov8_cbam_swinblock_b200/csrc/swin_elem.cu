@@ -134,7 +134,6 @@ __global__ void __launch_bounds__(256) swin_ln1_partition_vec_kernel(const T* __
                                                                     const float* __restrict__ beta, T* __restrict__ n1,
                                                                     float* __restrict__ mean, float* __restrict__ rstd,
                                                                     WinGeom g) {
-  pdl_enter();
   constexpr int VE = VecOf<T>::VE, N = NV * VE, TPW = 32 / LPT;
   const int lane = threadIdx.x & 31, l = lane % LPT, grp = lane / LPT;
   float gm[N], bt[N];
@@ -169,7 +168,6 @@ __global__ void __launch_bounds__(256) swin_res_ln2_vec_kernel(const T* __restri
                                                               const float* __restrict__ gamma, const float* __restrict__ beta,
                                                               T* __restrict__ y1, T* __restrict__ u, float* __restrict__ mean,
                                                               float* __restrict__ rstd, long long Ttok, int C) {
-  pdl_enter();
   constexpr int VE = VecOf<T>::VE, N = NV * VE, TPW = 32 / LPT;
   const int lane = threadIdx.x & 31, l = lane % LPT, grp = lane / LPT;
   float gm[N], bt[N];
@@ -203,7 +201,6 @@ __global__ void __launch_bounds__(256) swin_res_ln2_vec_kernel(const T* __restri
 template <typename T, int LPT, int NV, int MODE>
 __global__ void __launch_bounds__(256) swin_move_vec_kernel(const T* __restrict__ a, const T* __restrict__ b2, T* __restrict__ out,
                                                            WinGeom g) {
-  pdl_enter();
   constexpr int VE = VecOf<T>::VE, N = NV * VE, TPW = 32 / LPT;
   const int lane = threadIdx.x & 31, l = lane % LPT, grp = lane / LPT;
   const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -247,7 +244,6 @@ __global__ void __launch_bounds__(256) swin_ln_bwd_vec_kernel(const T* __restric
                                                              const T* __restrict__ gres, const float* __restrict__ gamma,
                                                              const float* __restrict__ mean, const float* __restrict__ rstd,
                                                              T* __restrict__ gin, float* __restrict__ part, WinGeom g) {
-  pdl_enter();
   constexpr int VE = VecOf<T>::VE, N = NV * VE, TPW = 32 / LPT;
   extern __shared__ float sm[];  // [warps][2][C]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
@@ -348,7 +344,6 @@ __global__ void __launch_bounds__(256) swin_ln1_partition_kernel(const T* __rest
                                                                 const float* __restrict__ beta, T* __restrict__ n1,
                                                                 float* __restrict__ mean, float* __restrict__ rstd,
                                                                 WinGeom g) {
-  pdl_enter();
   const int lane = threadIdx.x & 31;
   const long long t = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (t >= g.T) return;
@@ -377,7 +372,6 @@ __global__ void __launch_bounds__(256) swin_res_ln2_kernel(const T* __restrict__
                                                           const float* __restrict__ gamma, const float* __restrict__ beta,
                                                           T* __restrict__ y1, T* __restrict__ u, float* __restrict__ mean,
                                                           float* __restrict__ rstd, long long Ttok, int C) {
-  pdl_enter();
   const int lane = threadIdx.x & 31;
   const long long t = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (t >= Ttok) return;
@@ -416,7 +410,6 @@ __device__ __forceinline__ float gelu_erf_grad(float a) {
 template <typename T, bool BWD>
 __global__ void __launch_bounds__(256) swin_gelu_kernel(const T* __restrict__ a, const T* __restrict__ gh, T* __restrict__ out,
                                                        long long n) {
-  pdl_enter();
   constexpr int V = 16 / sizeof(T);
   const long long nv = n / V;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (long long)gridDim.x * blockDim.x) {
@@ -444,7 +437,6 @@ __global__ void __launch_bounds__(256) swin_gelu_kernel(const T* __restrict__ a,
 template <typename T>
 __global__ void __launch_bounds__(256) swin_res_reverse_kernel(const T* __restrict__ y1, const T* __restrict__ m,
                                                               T* __restrict__ out, WinGeom g) {
-  pdl_enter();
   const int lane = threadIdx.x & 31;
   const long long t = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (t >= g.T) return;
@@ -457,7 +449,6 @@ __global__ void __launch_bounds__(256) swin_res_reverse_kernel(const T* __restri
 // gy2[t,:] = g[b,y,x,:] for real tokens, 0 for padded ones (they are cropped, swin_block.py:58)
 template <typename T>
 __global__ void __launch_bounds__(256) swin_partition_kernel(const T* __restrict__ gsrc, const T* __restrict__ gadd, T* __restrict__ gtok, WinGeom g) {
-  pdl_enter();
   const int lane = threadIdx.x & 31;
   const long long t = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (t >= g.T) return;
@@ -482,7 +473,6 @@ __global__ void __launch_bounds__(256) swin_ln_bwd_kernel(const T* __restrict__ 
                                                          const float* __restrict__ mean, const float* __restrict__ rstd,
                                                          T* __restrict__ gin, float* __restrict__ part, WinGeom g,
                                                          int tokens_per_cta) {
-  pdl_enter();
   extern __shared__ float sm[];  // [warps][2][C]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
   const int C = g.C, npl = (C + 31) / 32;
@@ -543,7 +533,6 @@ __global__ void __launch_bounds__(256) swin_ln_bwd_kernel(const T* __restrict__ 
 // [rows][2][C] partials -> ggamma[C], gbeta[C]   (fixed order)
 __global__ void __launch_bounds__(1024) fold_ln_kernel(const float* __restrict__ part, float* __restrict__ gg, float* __restrict__ gb,
                                                        int rows, int C) {
-  pdl_enter();
   // 32 columns per block: lane = column, the block's 32 warps split the rows, fixed-order smem fold
   __shared__ float sm[32][33];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -563,7 +552,6 @@ __global__ void __launch_bounds__(1024) fold_ln_kernel(const float* __restrict__
 
 // out[i] = sum_r part[r][i]   (fixed order)
 __global__ void fold_rows_kernel(const float* __restrict__ part, float* __restrict__ out, int rows, int n) {
-  pdl_enter();
   __shared__ float sm[8][32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int i = blockIdx.x * 32 + lane;
@@ -585,7 +573,6 @@ template <typename T, int VEC> struct alignas(sizeof(T) * VEC) PackT { T e[VEC];
 template <typename T>
 __global__ void __launch_bounds__(256) colsum_partial_kernel(const T* __restrict__ a, float* __restrict__ part, long long rows,
                                                             int n, int rows_per_cta) {
-  pdl_enter();
   // blockIdx.x: 128-column strip (lane owns 4 columns), blockIdx.y: row slab; the 8 warps interleave the slab's rows
   __shared__ float sm[8][128];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -661,11 +648,11 @@ extern "C" B200_API int b200_swin_ln1_partition(const void* x, const float* gamm
     if (pick_vec<T>(C, &vec, &iters) && (((uintptr_t)x | (uintptr_t)n1) & 15) == 0) {
       const unsigned grid = capped_grid(g.T, 32 / vec);
       B200_DISPATCH_VEC({
-        launch_k(swin_ln1_partition_vec_kernel<T, VEC, ITERS>, grid, 256, 0, (cudaStream_t)stream, (const T*)x, gamma, beta, (T*)n1, mean, rstd, g);
+        swin_ln1_partition_vec_kernel<T, VEC, ITERS><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)x, gamma, beta, (T*)n1, mean, rstd, g);
         return check_launch("swin_ln1_partition");
       });
     }
-    launch_k(swin_ln1_partition_kernel<T>, warps_grid(g.T), 256, 0, (cudaStream_t)stream, (const T*)x, gamma, beta, (T*)n1, mean, rstd, g);
+    swin_ln1_partition_kernel<T><<<warps_grid(g.T), 256, 0, (cudaStream_t)stream>>>((const T*)x, gamma, beta, (T*)n1, mean, rstd, g);
     return check_launch("swin_ln1_partition");
   });
 }
@@ -680,12 +667,12 @@ extern "C" B200_API int b200_swin_res_ln2(const void* n1, const void* a, const f
     if (pick_vec<T>(C, &vec, &iters) && (((uintptr_t)n1 | (uintptr_t)a | (uintptr_t)y1 | (uintptr_t)u) & 15) == 0) {
       const unsigned grid = capped_grid(tokens, 32 / vec);
       B200_DISPATCH_VEC({
-        launch_k(swin_res_ln2_vec_kernel<T, VEC, ITERS>, grid, 256, 0, (cudaStream_t)stream, (const T*)n1, (const T*)a, gamma, beta, (T*)y1,
+        swin_res_ln2_vec_kernel<T, VEC, ITERS><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)n1, (const T*)a, gamma, beta, (T*)y1,
                                                                                        (T*)u, mean, rstd, tokens, C);
         return check_launch("swin_res_ln2");
       });
     }
-    launch_k(swin_res_ln2_kernel<T>, warps_grid(tokens), 256, 0, (cudaStream_t)stream, (const T*)n1, (const T*)a, gamma, beta, (T*)y1,
+    swin_res_ln2_kernel<T><<<warps_grid(tokens), 256, 0, (cudaStream_t)stream>>>((const T*)n1, (const T*)a, gamma, beta, (T*)y1,
                                                                                  (T*)u, mean, rstd, tokens, C);
     return check_launch("swin_res_ln2");
   });
@@ -701,8 +688,8 @@ extern "C" B200_API int b200_swin_gelu(const void* a, const void* gh, void* out,
     const unsigned cap = (unsigned)sm_count() * 16;
     if (grid > cap) grid = cap;
     if (grid == 0) grid = 1;
-    if (backward) launch_k(swin_gelu_kernel<T, true>, grid, 256, 0, (cudaStream_t)stream, (const T*)a, (const T*)gh, (T*)out, n);
-    else launch_k(swin_gelu_kernel<T, false>, grid, 256, 0, (cudaStream_t)stream, (const T*)a, nullptr, (T*)out, n);
+    if (backward) swin_gelu_kernel<T, true><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)a, (const T*)gh, (T*)out, n);
+    else swin_gelu_kernel<T, false><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)a, nullptr, (T*)out, n);
     return check_launch("swin_gelu");
   });
 }
@@ -717,11 +704,11 @@ extern "C" B200_API int b200_swin_res_reverse(const void* y1, const void* m, voi
     if (pick_vec<T>(C, &vec, &iters) && (((uintptr_t)y1 | (uintptr_t)m | (uintptr_t)out) & 15) == 0) {
       const unsigned grid = capped_grid(g.T, 32 / vec);
       B200_DISPATCH_VEC({
-        launch_k(swin_move_vec_kernel<T, VEC, ITERS, 0>, grid, 256, 0, (cudaStream_t)stream, (const T*)y1, (const T*)m, (T*)out, g);
+        swin_move_vec_kernel<T, VEC, ITERS, 0><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)y1, (const T*)m, (T*)out, g);
         return check_launch("swin_res_reverse");
       });
     }
-    launch_k(swin_res_reverse_kernel<T>, warps_grid(g.T), 256, 0, (cudaStream_t)stream, (const T*)y1, (const T*)m, (T*)out, g);
+    swin_res_reverse_kernel<T><<<warps_grid(g.T), 256, 0, (cudaStream_t)stream>>>((const T*)y1, (const T*)m, (T*)out, g);
     return check_launch("swin_res_reverse");
   });
 }
@@ -736,11 +723,11 @@ static int swin_partition_impl(const void* src, const void* add, void* tok, int3
     if (pick_vec<T>(C, &vec, &iters) && (((uintptr_t)src | (uintptr_t)add | (uintptr_t)tok) & 15) == 0) {
       const unsigned grid = capped_grid(g.T, 32 / vec);
       B200_DISPATCH_VEC({
-        launch_k(swin_move_vec_kernel<T, VEC, ITERS, 1>, grid, 256, 0, (cudaStream_t)stream, (const T*)src, (const T*)add, (T*)tok, g);
+        swin_move_vec_kernel<T, VEC, ITERS, 1><<<grid, 256, 0, (cudaStream_t)stream>>>((const T*)src, (const T*)add, (T*)tok, g);
         return check_launch("swin_partition");
       });
     }
-    launch_k(swin_partition_kernel<T>, warps_grid(g.T), 256, 0, (cudaStream_t)stream, (const T*)src, (const T*)add, (T*)tok, g);
+    swin_partition_kernel<T><<<warps_grid(g.T), 256, 0, (cudaStream_t)stream>>>((const T*)src, (const T*)add, (T*)tok, g);
     return check_launch("swin_partition");
   });
 }
@@ -784,11 +771,11 @@ extern "C" B200_API int b200_swin_ln_bwd(const void* gout, const void* xin, cons
         if (mode == 0) {
           auto k = swin_ln_bwd_vec_kernel<T, VEC, ITERS, 0>;
           cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-          launch_k(k, ctas, 256, smem, st, (const T*)gout, (const T*)xin, (const T*)gres, gamma, mean, rstd, (T*)gin, (float*)workspace, g);
+          k<<<ctas, 256, smem, st>>>((const T*)gout, (const T*)xin, (const T*)gres, gamma, mean, rstd, (T*)gin, (float*)workspace, g);
         } else {
           auto k = swin_ln_bwd_vec_kernel<T, VEC, ITERS, 1>;
           cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-          launch_k(k, ctas, 256, smem, st, (const T*)gout, (const T*)xin, nullptr, gamma, mean, rstd, (T*)gin, (float*)workspace, g);
+          k<<<ctas, 256, smem, st>>>((const T*)gout, (const T*)xin, nullptr, gamma, mean, rstd, (T*)gin, (float*)workspace, g);
         }
         return check_launch("swin_ln_bwd");
       });
@@ -796,16 +783,16 @@ extern "C" B200_API int b200_swin_ln_bwd(const void* gout, const void* xin, cons
     if (mode == 0) {
       auto k = swin_ln_bwd_kernel<T, 0>;
       cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      launch_k(k, ctas, 256, smem, st, (const T*)gout, (const T*)xin, (const T*)gres, gamma, mean, rstd, (T*)gin, (float*)workspace, g, kLnTokensPerCta);
+      k<<<ctas, 256, smem, st>>>((const T*)gout, (const T*)xin, (const T*)gres, gamma, mean, rstd, (T*)gin, (float*)workspace, g, kLnTokensPerCta);
     } else {
       auto k = swin_ln_bwd_kernel<T, 1>;
       cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      launch_k(k, ctas, 256, smem, st, (const T*)gout, (const T*)xin, nullptr, gamma, mean, rstd, (T*)gin, (float*)workspace, g, kLnTokensPerCta);
+      k<<<ctas, 256, smem, st>>>((const T*)gout, (const T*)xin, nullptr, gamma, mean, rstd, (T*)gin, (float*)workspace, g, kLnTokensPerCta);
     }
     return check_launch("swin_ln_bwd");
   });
   if (rc) return rc;
-  launch_k(fold_ln_kernel, (2 * C + 31) / 32, 1024, 0, st, (const float*)workspace, ggamma, gbeta, (int)ctas, C);
+  fold_ln_kernel<<<(2 * C + 31) / 32, 1024, 0, st>>>((const float*)workspace, ggamma, gbeta, (int)ctas, C);
   return check_launch("swin_ln_bwd_fold");
 }
 
@@ -840,10 +827,10 @@ extern "C" B200_API int b200_colsum(const void* a, float* out, void* workspace, 
       b200::set_error("colsum: n must be a multiple of 4 and the input %zu-byte aligned", 4 * sizeof(T));
       return B200_ERR_ALIGN;
     }
-    launch_k(colsum_partial_kernel<T>, dim3((n + 127) / 128, rblocks), 256, 0, st, (const T*)a, (float*)workspace, rows, n, rows_per);
+    colsum_partial_kernel<T><<<dim3((n + 127) / 128, rblocks), 256, 0, st>>>((const T*)a, (float*)workspace, rows, n, rows_per);
     return check_launch("colsum_partial");
   });
   if (rc) return rc;
-  launch_k(fold_rows_kernel, (n + 31) / 32, 256, 0, st, (const float*)workspace, out, (int)rblocks, n);
+  fold_rows_kernel<<<(n + 31) / 32, 256, 0, st>>>((const float*)workspace, out, (int)rblocks, n);
   return check_launch("colsum_fold");
 }

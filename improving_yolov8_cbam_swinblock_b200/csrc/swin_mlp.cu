@@ -149,7 +149,6 @@ __global__ void __launch_bounds__(kThreads, 1)
 swin_mlp_fwd_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmOut,
                     const __grid_constant__ CUtensorMap tmW1, const __grid_constant__ CUtensorMap tmW2,
                     const __grid_constant__ CUtensorMap tmH, MlpParams P) {
-  pdl_enter();
   using S = MlpSmem;
   extern __shared__ __align__(1024) unsigned char smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();   // 128-byte swizzle atoms need a 1024-byte aligned base: no slack is budgeted
@@ -496,7 +495,6 @@ swin_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_consta
                     const __grid_constant__ CUtensorMap tmW1, const __grid_constant__ CUtensorMap tmW2,
                     const __grid_constant__ CUtensorMap tmXhat, const __grid_constant__ CUtensorMap tmGa,
                     const __grid_constant__ CUtensorMap tmGy, MlpBwdParams P) {
-  pdl_enter();
   using S = MlpBwdSmem;
   extern __shared__ __align__(1024) unsigned char smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
@@ -830,7 +828,6 @@ swin_mlp_bwd_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_consta
 __global__ void swin_mlp_prep_kernel(const float* __restrict__ w1, const float* __restrict__ b1, const float* __restrict__ gamma,
                                      const float* __restrict__ beta, const float* __restrict__ w2, uint16_t* __restrict__ w1f,
                                      float* __restrict__ b1f, uint16_t* __restrict__ w2h, int C, int hid, int fmt) {
-  pdl_enter();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp < hid) {
     float acc = 0.f;
@@ -867,8 +864,8 @@ extern "C" B200_API int b200_swin_mlp_prep(const float* w1, const float* b1, con
   B200_REQUIRE(C > 0 && w1 && b1 && gamma && beta && w2 && w1f && b1f && w2h, B200_ERR_SHAPE, "swin_mlp_prep: null pointer / bad C");
   const int hid = 4 * C;
   const int threads = 256, blocks = (hid * 32 + threads - 1) / threads;
-  launch_k(tc::swin_mlp_prep_kernel, blocks, threads, 0, (cudaStream_t)stream, w1, b1, gamma, beta, w2, (uint16_t*)w1f, b1f, (uint16_t*)w2h, C, hid,
-                                                                           dtype == B200_BF16 ? 1 : 0);
+  tc::swin_mlp_prep_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(w1, b1, gamma, beta, w2, (uint16_t*)w1f, b1f, (uint16_t*)w2h, C, hid,
+                                                                         dtype == B200_BF16 ? 1 : 0);
   return check_launch("swin_mlp_prep");
 }
 
@@ -893,7 +890,7 @@ extern "C" B200_API int b200_swin_mlp_fwd(const void* y1, const void* w1f, const
   const int grid = P.n_tiles < sm_count() ? P.n_tiles : sm_count();
   auto kern = dtype == B200_BF16 ? swin_mlp_fwd_kernel<1> : swin_mlp_fwd_kernel<0>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, MlpSmem::TOTAL);
-  launch_k(kern, grid, kThreads, MlpSmem::TOTAL, (cudaStream_t)stream, *mY, *mO, *mW1, *mW2, *mH, P);
+  kern<<<grid, kThreads, MlpSmem::TOTAL, (cudaStream_t)stream>>>(*mY, *mO, *mW1, *mW2, *mH, P);
   return check_launch("swin_mlp_fwd");
 }
 
@@ -918,6 +915,6 @@ extern "C" B200_API int b200_swin_mlp_bwd(const void* gout, const void* y1, cons
   const int grid = P.n_tiles < sm_count() ? P.n_tiles : sm_count();
   auto kern = dtype == B200_BF16 ? swin_mlp_bwd_kernel<1> : swin_mlp_bwd_kernel<0>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, MlpBwdSmem::TOTAL);
-  launch_k(kern, grid, kThreads, MlpBwdSmem::TOTAL, (cudaStream_t)stream, *mY, *mG, *mW1, *mW2, *mX, *mGa, *mGy, P);
+  kern<<<grid, kThreads, MlpBwdSmem::TOTAL, (cudaStream_t)stream>>>(*mY, *mG, *mW1, *mW2, *mX, *mGa, *mGy, P);
   return check_launch("swin_mlp_bwd");
 }

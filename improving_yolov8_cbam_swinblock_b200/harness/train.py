@@ -10,7 +10,6 @@ SGD(momentum 0.937, nesterov) with the trainer's three parameter groups (trainer
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn as nn
@@ -98,15 +97,13 @@ class Trainer:
                 self._views.append(p.grad)
                 off += p.numel()
             # Autograd ACCUMULATES into an existing .grad (one add kernel per parameter and step, ~160 launches, plus the zero fill).
-            # Default: let the backward produce fresh gradients and move them into the flat buffer with ONE multi-tensor copy
-            # (B200_FLAT_COPY=0: the accumulate-in-place form).
-            self._flat_copy = os.environ.get("B200_FLAT_COPY", "1") != "0"
+            # Instead the backward produces fresh gradients and ONE multi-tensor copy moves them into the flat buffer.
         # SURVEY 8(f)-3: under autocast every stock convolution casts its f32 weight to the compute dtype in the forward and its
         # 16-bit weight gradient back to f32 in the backward -- two tiny kernels per layer and step (~100 launches).  Instead: one
         # 16-bit leaf per layer, all refreshed by ONE multi-tensor copy at the start of the step and all gradients copied back by
         # ONE multi-tensor copy after the backward.  Same values as autocast's casts (bit-identical step).
         self._w16 = []   # (Conv module, f32 parameter, 16-bit leaf, f32 gradient buffer)
-        if self.device.type == "cuda" and amp_dtype in (torch.bfloat16, torch.float16) and os.environ.get("B200_W16", "1") != "0":
+        if self.device.type == "cuda" and amp_dtype in (torch.bfloat16, torch.float16):
             for m_ in model.modules():
                 if isinstance(m_, graph.Conv) and m_.conv_fn is None and m_.conv.bias is None and m_.conv.weight.requires_grad \
                         and m_.conv.padding_mode == "zeros":
@@ -140,11 +137,8 @@ class Trainer:
 
     def _fwd_bwd(self, dev_batch):
         if self._flat is not None:
-            if self._flat_copy:
-                for p in self._params:
-                    p.grad = None           # fresh gradients from the backward, gathered into the flat buffer below
-            else:
-                self._flat.zero_()          # grads are views of the flat buffer: autograd accumulates in place
+            for p in self._params:
+                p.grad = None               # fresh gradients from the backward, gathered into the flat buffer below
         if self._w16:
             with torch.no_grad():
                 torch._foreach_copy_([t[2] for t in self._w16], [t[1] for t in self._w16])   # f32 weights -> 16-bit leaves
@@ -158,7 +152,7 @@ class Trainer:
                 torch._foreach_copy_([t[3] for t in live], [t[2].grad for t in live])       # 16-bit gradients -> f32 .grad
             for _, p, _, g32 in live:
                 p.grad = g32
-        if self._flat is not None and self._flat_copy:
+        if self._flat is not None:
             src, dst, missing = [], [], []
             for p, v in zip(self._params, self._views):
                 if p.grad is None:
@@ -212,31 +206,16 @@ class Trainer:
                     self._static_items = self._fwd_bwd(self._static)
                     self._update()
             else:
-                # thread_local: the NCCL watchdog thread may make CUDA calls while this thread captures
-                # opt-in: capturing the NCCL all-reduce into the same graph measured no faster at N=2 (20.7-21.3 vs 20.4 ms/step) and a
-                # graph that holds NCCL kernels must be destroyed before the communicator (release_graphs) -- default: two graphs
-                one = os.environ.get("B200_ALLREDUCE_IN_GRAPH", "0") == "1"
-                if one:
-                    try:   # ONE graph: forward + loss + backward, the NCCL all-reduce of the flat buffer, clip + SGD
-                        with torch.cuda.graph(ga, capture_error_mode="thread_local"):
-                            self._static_items = self._fwd_bwd(self._static)
-                            self._exchange()
-                            self._update()
-                        self._graph_mode = "one graph (all-reduce captured)"
-                    except Exception as e:  # noqa: BLE001  a backend that cannot capture collectives: two graphs around an eager all-reduce
-                        self._graph_error = f"all-reduce capture failed: {type(e).__name__}: {e}"
-                        torch.cuda.synchronize(self.device)
-                        ga = torch.cuda.CUDAGraph()
-                        one = False
-                if not one:
-                    gb = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(ga, capture_error_mode="thread_local"):
-                        self._static_items = self._fwd_bwd(self._static)
-                    self._exchange()
-                    with torch.cuda.graph(gb, pool=ga.pool(), capture_error_mode="thread_local"):
-                        self._update()
-                    self._graph_b = gb
-                    self._graph_mode = "two graphs around an eager all-reduce"
+                # thread_local: the NCCL watchdog thread may make CUDA calls while this thread captures.  The all-reduce stays
+                # outside the graphs: capturing it too measured no faster at N=2 (20.7-21.3 vs 20.4 ms/step)
+                gb = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(ga, capture_error_mode="thread_local"):
+                    self._static_items = self._fwd_bwd(self._static)
+                self._exchange()
+                with torch.cuda.graph(gb, pool=ga.pool(), capture_error_mode="thread_local"):
+                    self._update()
+                self._graph_b = gb
+                self._graph_mode = "two graphs around an eager all-reduce"
             self._graph = ga
         except Exception as e:  # noqa: BLE001  capture is an optimisation; eager launches remain correct
             self._graph, self._graph_b, self._graph_error = None, None, f"{type(e).__name__}: {e}"
@@ -244,8 +223,8 @@ class Trainer:
         return self._graph is not None
 
     def release_graphs(self):
-        """Destroy the captured graphs (they hold NCCL kernels when the all-reduce was captured: the communicator must not be
-        torn down while such a graph exists) and fall back to eager launches."""
+        """Destroy the captured graphs and fall back to eager launches.  The graphs hold no NCCL kernels (the all-reduce runs
+        eagerly between them), so the communicator does not depend on them."""
         self._graph, self._graph_b, self._static_items = None, None, None
         if self.device.type == "cuda":
             import gc

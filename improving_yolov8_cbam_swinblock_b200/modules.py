@@ -14,8 +14,6 @@ carrying real data raises, and on CUDA a missing ``libb200yolo.so`` raises.
 """
 from __future__ import annotations
 
-import os
-
 import torch
 import torch.nn as nn
 
@@ -228,5 +226,3 @@ BLOCKS = {"CBAM": CBAM, "SwinBlock": SwinBlock, "SPPF": SPPF, "conv_epilogue": c
           "concat": Fb.nhwc_concat, "chunk": Fb.nhwc_chunk, "input_prep": Fb.u8_to_nhwc, "cls_loss": Fb.cls_bce_sum,
           "upsample": Fb.nhwc_upsample_nearest, "head_conv": Fb.head_conv, "det_loss": Fb.DetLossKernels, "stem_conv": Fb.stem_conv, "conv3x3": Fb.conv3x3,
           "fork": Fb.nhwc_fork}
-if os.environ.get("B200_FORK", "1") == "0":   # A/B switch: autograd's own gradient accumulation at the fan-out points
-    BLOCKS.pop("fork")

@@ -184,19 +184,21 @@ def test_whole_model_bf16_vs_oracle_blocks():
     assert (num / den) ** 0.5 <= 1.25 * (num16 / den) ** 0.5 + 1e-2, ((num / den) ** 0.5, (num16 / den) ** 0.5)
 
 
-def test_weight_leaves_step_is_bit_identical_to_autocast_casts(monkeypatch):
+def test_weight_leaves_step_is_bit_identical_to_leafless_trainer():
     """The Trainer hands every stock convolution a 16-bit leaf copy of its weight (one multi-tensor refresh per step, one
     multi-tensor copy of the gradients back) instead of autocast's per-layer cast kernels: same values, so three steps must
-    leave bit-identical parameters and loss items (cuDNN deterministic, same algorithms for the same shapes)."""
+    leave bit-identical parameters and loss items (cuDNN deterministic, same algorithms for the same shapes).  The
+    reference trainer has its leaves taken away, so its convolutions go through autocast's casts."""
     import improving_yolov8_cbam_swinblock_b200 as P
     from improving_yolov8_cbam_swinblock_b200.harness import synthetic, train
 
     torch.backends.cudnn.deterministic = True
     try:
-        monkeypatch.setenv("B200_W16", "1")
         a = train.Trainer(P.BLOCKS, "n", 80, device="cuda:0", amp_dtype=torch.bfloat16, seed=5)
-        monkeypatch.setenv("B200_W16", "0")
         b = train.Trainer(P.BLOCKS, "n", 80, device="cuda:0", amp_dtype=torch.bfloat16, seed=5)
+        for m, *_ in b._w16:
+            m.w16 = None
+        b._w16 = []
         assert len(a._w16) > 30 and not b._w16
         for t in (a, b):
             t.max_boxes = synthetic.BOXES_PER_IMAGE
