@@ -4,8 +4,8 @@ Caller-side code (SURVEY section 2.1 marks ``utils/loss.py:152-255`` / ``utils/t
 the training harness"; the reference package cannot travel to the GPU box, so this is a dense restatement).
 It computes the same function as ``v8DetectionLoss.__call__`` + ``TaskAlignedAssigner.forward`` but with
 mask-multiplies instead of boolean indexing and no ``.item()``-style host syncs, so one training step can
-be enqueued without the host waiting on the device.  tests/test_harness_vs_reference.py checks the three loss
-components against the reference on CPU.
+be enqueued without the host waiting on the device.  tests/test_det_loss_oracle.py checks the assigner and the three loss
+components on CPU against oracle/det_loss.py, a line-by-line restatement of the reference that shares no code with this one.
 """
 from __future__ import annotations
 

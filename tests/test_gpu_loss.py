@@ -63,7 +63,8 @@ def _gt(bs, nmax, imgsz, nc, seed, empty_image=True):
     return out.cuda()
 
 
-CASES = [(3, 80, [(16, 16), (8, 8), (4, 4)], 128, 5), (4, 80, [(80, 80), (40, 40), (20, 20)], 640, 8), (2, 16, [(12, 20)], 160, 3)]
+CASES = [(3, 80, [(16, 16), (8, 8), (4, 4)], 128, 5), (4, 80, [(80, 80), (40, 40), (20, 20)], 640, 8), (2, 16, [(12, 20)], 160, 3),
+         (2, 16, [(32, 32), (16, 16), (8, 8), (4, 4)], 128, 4), (2, 8, [(12, 20), (6, 10), (3, 5)], 96, 4)]
 
 
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16, torch.float32])
@@ -90,8 +91,10 @@ def test_det_decode_matches_torch(dtype, bs, nc, sizes, imgsz, nmax):
 @pytest.mark.parametrize("bs,nc,sizes,imgsz,nmax", CASES)
 @pytest.mark.parametrize("spread", [1.0, 3.0])
 def test_tal_assign_matches_the_torch_restatement(bs, nc, sizes, imgsz, nmax, spread):
-    """tal.py:41-327 as restated in harness/loss.py:task_aligned_assign (pinned against the reference on CPU by
-    tests/test_harness_vs_reference.py), on the same decoded boxes / scores: identical targets wherever the target is non-zero."""
+    """tal.py:41-327 as restated in harness/loss.py:task_aligned_assign (pinned against the restated reference, oracle/det_loss.py,
+    by tests/test_det_loss_oracle.py), on the same decoded boxes / scores: identical targets wherever either target is non-zero.
+    The kernel copies the restatement's f32 arithmetic, so only an exact metric tie at a GT's k-th place (torch.topk orders
+    ties arbitrarily, the kernel takes the lower anchor index) could separate them; these random inputs have none."""
     from improving_yolov8_cbam_swinblock_b200 import functional as Fb
     from improving_yolov8_cbam_swinblock_b200.harness import loss as hl
     from improving_yolov8_cbam_swinblock_b200.harness.graph import make_anchors
@@ -108,11 +111,9 @@ def test_tal_assign_matches_the_torch_restatement(bs, nc, sizes, imgsz, nmax, sp
     pos = (wv > 0) | (tval > 0)
     assert int(pos.sum()) > 5 * bs
     mism = (tval - wv).abs() > 1e-6 * wv.abs().clamp(min=1e-3)
-    assert int(mism.sum()) <= 0.002 * int(pos.sum()) + 1, f"{int(mism.sum())} of {int(pos.sum())} positives differ"
-    ok = pos & ~mism
-    assert torch.equal(tlabel[ok].long(), wl[ok])
-    torch.testing.assert_close(tbox[ok], (wb / st)[ok], rtol=1e-6, atol=1e-6)
-    assert float((tval.sum() - wv.sum()).abs()) <= 1e-3 * float(wv.sum())
+    assert int(mism.sum()) == 0, f"{int(mism.sum())} of {int(pos.sum())} positives differ"
+    assert torch.equal(tlabel[pos].long(), wl[pos])
+    assert torch.equal(tbox[pos], (wb / st)[pos])
     # run-to-run identical
     t2 = Fb.tal_assign(pred, scores, gt, [f.shape[2:] for f in box], strides)
     assert torch.equal(t2[0], tlabel) and torch.equal(t2[1], tval) and torch.equal(t2[2], tbox)

@@ -1,6 +1,8 @@
 """CPU: the harness' caller-side graph and loss compute the same function as the reference's DetectionModel +
 v8DetectionLoss on identical weights, against the stored fixture ``tests/golden/model/detection_n_256.npz``
-(``python -m oracle.make_golden model``).  The plugin tests below drive the reference package itself and run only where it
+(``python -m oracle.make_golden model``).  The committed fixture has ``source = "harness"``: the harness produced it where the
+reference was absent, so for the loss it shows only that the harness still computes what it computed then.  What pins the loss
+to the reference's function is tests/test_det_loss_oracle.py (oracle/det_loss.py).  The plugin tests below drive the reference package itself and run only where it
 is importable (``oracle/_ref``, made by ``oracle/build_ref.py``); the repository does not ship it."""
 import os
 

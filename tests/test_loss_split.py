@@ -1,6 +1,6 @@
 """CPU: the harness loss on the Detect head's un-concatenated (box, cls) maps with (label, value) targets -- the form the fused
-classification-loss kernel consumes (SURVEY 8(f)-4) -- equals the dense form (which tests/test_harness_vs_reference.py pins
-against the reference's v8DetectionLoss)."""
+classification-loss kernel consumes (SURVEY 8(f)-4) -- equals the dense form.  Both forms are pinned to the reference's v8DetectionLoss by
+tests/test_det_loss_oracle.py, against the line-by-line restatement oracle/det_loss.py."""
 import torch
 import torch.nn.functional as F
 
