@@ -11,7 +11,9 @@
 //   qkv  [T, 3C]  packed rows (q | k | v) as produced by the in_proj GEMM (+bias)
 //   o    [T, C]   heads concatenated
 //   lse  [T, nh]  f32 log-sum-exp of the scaled scores (saved for the backward)
-#include "common.cuh"
+// BIAS (SwinBlockRPB): the dense relative-position bias [nh][64][64] (swin_rpb.cu) is added to the scores before the
+// mask; the backward also writes each CTA's unscaled dS = p (dP - delta) to its own workspace slot [win][h][64][64].
+#include "swin_rpb.cuh"
 
 namespace b200 {
 namespace {
@@ -20,9 +22,9 @@ constexpr int LMAX = 64;
 
 template <typename T> __device__ __forceinline__ float ldf(const T* p) { return DT<T>::to_f(*p); }
 
-template <typename T>
+template <typename T, bool BIAS>
 __global__ void __launch_bounds__(LMAX) swin_attn_fwd_kernel(const T* __restrict__ qkv, T* __restrict__ o, float* __restrict__ lse,
-                                                             int L, int C, int nh, const ShiftMask M) {
+                                                             int L, int C, int nh, const ShiftMask M, const float* __restrict__ bias) {
   extern __shared__ __align__(16) float sm[];
   const int hd = C / nh, hp = hd + 4;
   float* ks = sm;             // [L][hp]
@@ -53,6 +55,12 @@ __global__ void __launch_bounds__(LMAX) swin_attn_fwd_kernel(const T* __restrict
         s[j] += q0 * kv.x + q1 * kv.y + q2 * kv.z + q3 * kv.w;
       }
   }
+  if constexpr (BIAS) {
+    const float* brow = bias + ((size_t)h * 64 + i) * 64;
+#pragma unroll
+    for (int j = 0; j < LMAX; ++j)
+      if (j < L) s[j] += brow[j];
+  }
   const unsigned long long allowed = allowed_keys(M, win, i);   // shifted-window mask (all ones when shift == 0)
   float m = -INFINITY;
 #pragma unroll
@@ -82,10 +90,11 @@ __global__ void __launch_bounds__(LMAX) swin_attn_fwd_kernel(const T* __restrict
 }
 
 // backward: gqkv [T,3C] from qkv, o, lse and go [T,C]   (SURVEY App. A.3 "Attention")
-template <typename T>
+template <typename T, bool BIAS>
 __global__ void __launch_bounds__(LMAX) swin_attn_bwd_kernel(const T* __restrict__ qkv, const T* __restrict__ o,
                                                              const float* __restrict__ lse, const T* __restrict__ go,
-                                                             T* __restrict__ gqkv, int L, int C, int nh, const ShiftMask M) {
+                                                             T* __restrict__ gqkv, int L, int C, int nh, const ShiftMask M,
+                                                             const float* __restrict__ bias, float* __restrict__ dws) {
   extern __shared__ __align__(16) float sm[];
   const int hd = C / nh, hp = hd + 4, lp = L + 1;
   float* b0 = sm;               // phase 1: K rows     phase 2: dO rows
@@ -129,6 +138,12 @@ __global__ void __launch_bounds__(LMAX) swin_attn_bwd_kernel(const T* __restrict
     }
     const float l = lse[(t0 + i) * nh + h];
     const unsigned long long allowed = allowed_keys(M, win, i);
+    if constexpr (BIAS) {
+      const float* brow = bias + ((size_t)h * 64 + i) * 64;
+#pragma unroll
+      for (int j = 0; j < LMAX; ++j)
+        if (j < L) s[j] += brow[j];
+    }
 #pragma unroll
     for (int j = 0; j < LMAX; ++j)
       if (j < L) {
@@ -136,6 +151,7 @@ __global__ void __launch_bounds__(LMAX) swin_attn_bwd_kernel(const T* __restrict
         const float dsj = p * (dp[j] - delta) * scale;
         ps[i * lp + j] = p;
         ds[i * lp + j] = dsj;
+        if constexpr (BIAS) dws[((size_t)win * nh + h) * 4096 + i * 64 + j] = p * (dp[j] - delta);
         s[j] = dsj;
       }
     // dQ[i,:] = sum_j dS[i,j] K[j,:]
@@ -190,6 +206,36 @@ int check_attn(int64_t tokens, int L, int C, int nh) {
   return B200_OK;
 }
 
+template <bool BIAS>
+int launch_attn_fwd(const void* qkv, const float* bias, void* o, float* lse, int64_t tokens, int L, int C, int nh, const ShiftMask& M,
+                    int dtype, cudaStream_t st) {
+  const int hd = C / nh;
+  const size_t smem = (size_t)2 * L * (hd + 4) * sizeof(float);
+  B200_REQUIRE(smem <= (size_t)max_smem_optin(), B200_ERR_UNSUPPORTED, "swin_attn_fwd: head dim %d too large", hd);
+  const unsigned grid = (unsigned)(tokens / L * nh);
+  return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
+    auto k = swin_attn_fwd_kernel<T, BIAS>;
+    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    k<<<grid, LMAX, smem, st>>>((const T*)qkv, (T*)o, lse, L, C, nh, M, bias);
+    return check_launch("swin_attn_fwd");
+  });
+}
+
+template <bool BIAS>
+int launch_attn_bwd(const void* qkv, const void* o, const float* lse, const void* go, const float* bias, void* gqkv, float* dws,
+                    int64_t tokens, int L, int C, int nh, const ShiftMask& M, int dtype, cudaStream_t st) {
+  const int hd = C / nh;
+  const size_t smem = ((size_t)2 * L * (hd + 4) + (size_t)2 * L * (L + 1)) * sizeof(float);
+  B200_REQUIRE(smem <= (size_t)max_smem_optin(), B200_ERR_UNSUPPORTED, "swin_attn_bwd: head dim %d too large", hd);
+  const unsigned grid = (unsigned)(tokens / L * nh);
+  return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
+    auto k = swin_attn_bwd_kernel<T, BIAS>;
+    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    k<<<grid, LMAX, smem, st>>>((const T*)qkv, (const T*)o, lse, (const T*)go, (T*)gqkv, L, C, nh, M, bias, dws);
+    return check_launch("swin_attn_bwd");
+  });
+}
+
 }  // namespace
 }  // namespace b200
 
@@ -202,16 +248,7 @@ extern "C" B200_API int b200_swin_attn_fwd(const void* qkv, void* o, float* lse,
   if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
   const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
   B200_REQUIRE(qkv && o, B200_ERR_SHAPE, "swin_attn_fwd: null pointer");
-  const int hd = C / nh;
-  const size_t smem = (size_t)2 * L * (hd + 4) * sizeof(float);
-  B200_REQUIRE(smem <= (size_t)max_smem_optin(), B200_ERR_UNSUPPORTED, "swin_attn_fwd: head dim %d too large", hd);
-  const unsigned grid = (unsigned)(tokens / L * nh);
-  return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
-    auto k = swin_attn_fwd_kernel<T>;
-    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k<<<grid, LMAX, smem, (cudaStream_t)stream>>>((const T*)qkv, (T*)o, lse, L, C, nh, M);
-    return check_launch("swin_attn_fwd");
-  });
+  return launch_attn_fwd<false>(qkv, nullptr, o, lse, tokens, L, C, nh, M, dtype, (cudaStream_t)stream);
 }
 
 extern "C" B200_API int b200_swin_attn_bwd(const void* qkv, const void* o, const float* lse, const void* go, void* gqkv,
@@ -221,14 +258,35 @@ extern "C" B200_API int b200_swin_attn_bwd(const void* qkv, const void* o, const
   if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
   const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
   B200_REQUIRE(qkv && o && lse && go && gqkv, B200_ERR_SHAPE, "swin_attn_bwd: null pointer");
-  const int hd = C / nh;
-  const size_t smem = ((size_t)2 * L * (hd + 4) + (size_t)2 * L * (L + 1)) * sizeof(float);
-  B200_REQUIRE(smem <= (size_t)max_smem_optin(), B200_ERR_UNSUPPORTED, "swin_attn_bwd: head dim %d too large", hd);
-  const unsigned grid = (unsigned)(tokens / L * nh);
-  return B200_DISPATCH_DTYPE(dtype, [&]() -> int {
-    auto k = swin_attn_bwd_kernel<T>;
-    cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k<<<grid, LMAX, smem, (cudaStream_t)stream>>>((const T*)qkv, (const T*)o, lse, (const T*)go, (T*)gqkv, L, C, nh, M);
-    return check_launch("swin_attn_bwd");
-  });
+  return launch_attn_bwd<false>(qkv, o, lse, go, nullptr, gqkv, nullptr, tokens, L, C, nh, M, dtype, (cudaStream_t)stream);
+}
+
+extern "C" B200_API int b200_swin_attn_fwd_rpb(const void* qkv, const float* bias, void* o, float* lse, int64_t tokens, int32_t L,
+                                               int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift,
+                                               int32_t dtype, void* stream) {
+  if (int rc = check_attn(tokens, L, C, nh)) return rc;
+  if (int rc = check_rpb(L, ws)) return rc;
+  if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
+  const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
+  B200_REQUIRE(qkv && bias && o, B200_ERR_SHAPE, "swin_attn_fwd_rpb: null pointer");
+  return launch_attn_fwd<true>(qkv, bias, o, lse, tokens, L, C, nh, M, dtype, (cudaStream_t)stream);
+}
+
+extern "C" B200_API int b200_swin_attn_bwd_rpb(const void* qkv, const void* o, const float* lse, const void* go, const float* bias,
+                                               void* gqkv, float* gtable, int32_t table_rows, void* workspace, size_t workspace_bytes,
+                                               int64_t tokens, int32_t L, int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws,
+                                               int32_t shift, int32_t dtype, void* stream) {
+  if (int rc = check_attn(tokens, L, C, nh)) return rc;
+  if (int rc = check_rpb(L, ws)) return rc;
+  if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
+  const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
+  B200_REQUIRE(table_rows == (2 * ws - 1) * (2 * ws - 1), B200_ERR_SHAPE, "swin_attn_bwd_rpb: table has %d rows, ws %d needs %d",
+               table_rows, ws, (2 * ws - 1) * (2 * ws - 1));
+  B200_REQUIRE(qkv && o && lse && go && bias && gqkv && gtable && workspace, B200_ERR_SHAPE, "swin_attn_bwd_rpb: null pointer");
+  const long long nslots = tokens / L;
+  B200_REQUIRE(workspace_bytes >= rpb_workspace_bytes(nslots, nh), B200_ERR_WORKSPACE, "swin_attn_bwd_rpb: workspace %zu < %zu bytes",
+               workspace_bytes, rpb_workspace_bytes(nslots, nh));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = launch_attn_bwd<true>(qkv, o, lse, go, bias, gqkv, (float*)workspace, tokens, L, C, nh, M, dtype, st)) return rc;
+  return rpb_fold((const float*)workspace, nslots, nh, ws, gtable, st);
 }

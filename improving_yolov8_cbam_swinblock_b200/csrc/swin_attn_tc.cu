@@ -11,13 +11,21 @@
 //   warps tcgen05.ld O, multiply by 1/rowsum, store the L real rows to o[T,C]; lse saved for the backward
 // Persistent CTAs (one per SM), 6 warps: 0-3 softmax/epilogue (TMEM lane quadrant = warp), 4 TMA producer, 5 MMA
 // issuer.  With HD = 64 everything is double-buffered so S(k+1) is computed while softmax(k) runs.
+// BIAS (SwinBlockRPB): the softmax threads add the dense relative-position bias row [h][i][0..64) (swin_rpb.cu) times log2(e)
+// to the scaled scores; the backward's threads add their row of unscaled dS into a workspace row only they own.  Nothing
+// else of either kernel changes: no shared memory, barrier, TMA or MMA is added.
 #include "tc.cuh"
+#include "swin_rpb.cuh"
 
 namespace b200 {
 namespace tc {
 namespace {
 
 constexpr int kThreads10 = 320;   // 8 softmax/epilogue warps + TMA warp + MMA warp
+constexpr float kLog2e = 1.4426950408889634f;
+
+__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" :: "l"(p)); }
+__device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 
 struct AttnParams {
   void* o;
@@ -26,6 +34,7 @@ struct AttnParams {
   int L, C, nh, n_items, n_pairs, fmt;
   float scale_log2;
   ShiftMask mask;
+  const float* bias;   // BIAS: dense [nh][64][64]
 };
 
 template <int HD> struct ACfg {
@@ -48,7 +57,7 @@ __device__ __forceinline__ uint32_t pack2f(float lo, float hi, int fmt) {
   return *reinterpret_cast<uint32_t*>(&p);
 }
 
-template <int HD>
+template <int HD, bool BIAS>
 __global__ void __launch_bounds__(kThreads10, 1) swin_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmO, AttnParams P) {
   using Cfg = ACfg<HD>;
   constexpr int KB = Cfg::KB, STAGES = Cfg::STAGES;
@@ -200,6 +209,11 @@ __global__ void __launch_bounds__(kThreads10, 1) swin_attn_fwd_tc_kernel(const _
       const int win = itc / P.nh, h = itc - win * P.nh;
       const long long tok = (long long)win * P.L + i;
       const unsigned long long allowed = allowed_keys(P.mask, win, i);   // shifted-window mask (all ones when shift == 0)
+      const float* brow = nullptr;
+      if constexpr (BIAS) {
+        brow = P.bias + ((size_t)h * 64 + i) * 64;
+        prefetch_l1(brow); prefetch_l1(brow + 32);
+      }
       mbar_wait(&s_full[s], ph);
       fence_after_sync();
       uint32_t v[32], w[32];
@@ -207,10 +221,18 @@ __global__ void __launch_bounds__(kThreads10, 1) swin_attn_fwd_tc_kernel(const _
       tmem_ld32(tS(s) + lane_sel + r * 64 + 32, w);
       tmem_ld_wait();
       float m = -INFINITY;
+      float4 ba4, bb4;
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
-        const float a = (j < P.L && ((allowed >> j) & 1ull)) ? __uint_as_float(v[j]) * P.scale_log2 : -INFINITY;
-        const float b = (j + 32 < P.L && ((allowed >> (j + 32)) & 1ull)) ? __uint_as_float(w[j]) * P.scale_log2 : -INFINITY;
+        float ba = 0.f, bb = 0.f;
+        if constexpr (BIAS) {
+          if ((j & 3) == 0) { ba4 = ldg4(brow + j); bb4 = ldg4(brow + 32 + j); }
+          ba = (&ba4.x)[j & 3] * kLog2e; bb = (&bb4.x)[j & 3] * kLog2e;
+        }
+        const float a = (j < P.L && ((allowed >> j) & 1ull))
+                            ? (BIAS ? fmaf(__uint_as_float(v[j]), P.scale_log2, ba) : __uint_as_float(v[j]) * P.scale_log2) : -INFINITY;
+        const float b = (j + 32 < P.L && ((allowed >> (j + 32)) & 1ull))
+                            ? (BIAS ? fmaf(__uint_as_float(w[j]), P.scale_log2, bb) : __uint_as_float(w[j]) * P.scale_log2) : -INFINITY;
         v[j] = __float_as_uint(a); w[j] = __float_as_uint(b);
         m = fmaxf(m, fmaxf(a, b));
       }
@@ -298,19 +320,20 @@ __global__ void __launch_bounds__(kThreads10, 1) swin_attn_fwd_tc_kernel(const _
   if (warp == 9) { fence_after_sync(); tmem_dealloc(tmem_base, Cfg::TMEM_COLS); }
 }
 
-template <int HD>
-int launch_fwd(const void* qkv, void* o, float* lse, long long T, int L, int C, int nh, const ShiftMask& M, int dtype, cudaStream_t st) {
+template <int HD, bool BIAS>
+int launch_fwd(const void* qkv, const float* bias, void* o, float* lse, long long T, int L, int C, int nh, const ShiftMask& M, int dtype,
+               cudaStream_t st) {
   using Cfg = ACfg<HD>;
   const CUtensorMap* m = tensor_map_2d(qkv, (uint64_t)T, (uint64_t)3 * C, (uint64_t)3 * C, (uint32_t)L, 64, dtype);
   const CUtensorMap* mo = tensor_map_2d(o, (uint64_t)T, (uint64_t)C, (uint64_t)C, (uint32_t)L, 64, dtype);
   if (!m || !mo) return B200_ERR_LAUNCH;
   AttnParams P;
-  P.o = o; P.lse = lse; P.T = T; P.L = L; P.C = C; P.nh = nh; P.mask = M;
+  P.o = o; P.lse = lse; P.T = T; P.L = L; P.C = C; P.nh = nh; P.mask = M; P.bias = bias;
   P.n_items = (int)(T / L) * nh;
   P.n_pairs = (P.n_items + 1) / 2;
   P.fmt = dtype == B200_BF16 ? 1 : 0;
   P.scale_log2 = 1.4426950408889634f / sqrtf((float)HD);
-  auto k = swin_attn_fwd_tc_kernel<HD>;
+  auto k = swin_attn_fwd_tc_kernel<HD, BIAS>;
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::TOTAL);
   int grid = P.n_pairs < sm_count() ? P.n_pairs : sm_count();
   k<<<grid, kThreads10, Cfg::TOTAL, st>>>(*m, *mo, P);
@@ -333,6 +356,8 @@ struct AttnBwdParams {
   int L, C, nh, n_items, n_pairs, fmt;
   float scale_log2, scale;
   ShiftMask mask;
+  const float* bias;   // BIAS: dense [nh][64][64]
+  float* dws;          // BIAS: dS slots [gridDim.x][warp group][item slot r][nh][64][64], zeroed before the launch
 };
 
 template <int HD> struct BCfg {
@@ -361,7 +386,7 @@ template <int HD> struct BCfg {
   static constexpr int TMEM_COLS = 512;
 };
 
-template <int HD>
+template <int HD, bool BIAS>
 __global__ void __launch_bounds__(kThreads10, 1)
 swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmGO,
                         const __grid_constant__ CUtensorMap tmOut, AttnBwdParams P) {
@@ -547,6 +572,14 @@ swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
       const long long tok = (long long)win * P.L + i;
       const unsigned long long allowed = allowed_keys(P.mask, win, i);   // shifted-window mask (all ones when shift == 0)
       const float lraw = valid ? P.lse[tok * P.nh + h] : 0.f;   // consumed after the wait below: the load latency hides behind it
+      const float* brow = nullptr;
+      float* wrow = nullptr;
+      if constexpr (BIAS) {
+        brow = P.bias + ((size_t)h * 64 + i) * 64;
+        wrow = P.dws + ((((size_t)blockIdx.x * 2 + g) * 2 + r) * P.nh + h) * 4096 + i * 64;
+        prefetch_l1(brow); prefetch_l1(brow + 32);
+        if (valid) { prefetch_l1(wrow); prefetch_l1(wrow + 32); }
+      }
       mbar_wait(&sdp_full[s], ph);
       fence_after_sync();
       const float l2 = lraw * 1.4426950408889634f;
@@ -559,10 +592,19 @@ swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
         tmem_ld32(tS(s) + lane_sel + r * 64 + hf * 32, sh);
         tmem_ld32(tDP(s) + lane_sel + r * 64 + hf * 32, dv);
         tmem_ld_wait();
+        float4 b4;
 #pragma unroll
         for (int jj = 0; jj < 32; ++jj) {
           const int j = hf * 32 + jj;
-          const float p = (j < P.L && valid && ((allowed >> j) & 1ull)) ? exp2f(__uint_as_float(sh[jj]) * P.scale_log2 - l2) : 0.f;
+          float bj = 0.f;
+          if constexpr (BIAS) {
+            if ((jj & 3) == 0) b4 = ldg4(brow + j);
+            bj = (&b4.x)[jj & 3] * kLog2e;
+          }
+          const float p = (j < P.L && valid && ((allowed >> j) & 1ull))
+                              // with bias one fma, like the contracted s * c - l2 of the bias-free path: a zero table is bit-exact
+                              ? exp2f(BIAS ? fmaf(__uint_as_float(sh[jj]), P.scale_log2, bj - l2) : __uint_as_float(sh[jj]) * P.scale_log2 - l2)
+                              : 0.f;
           sh[jj] = __float_as_uint(p);
           delta += p * __uint_as_float(dv[jj]);
         }
@@ -587,6 +629,7 @@ swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
         for (int cc = 0; cc < 4; ++cc) {
           const int c = hf * 4 + cc;
           uint32_t pw[4], dw[4];
+          float gs[8];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
             const int jj = cc * 8 + 2 * e;
@@ -596,6 +639,19 @@ swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
             // the next pair's V tile
             dw[e] = valid ? pack2f(p0 * (__uint_as_float(dv[jj]) - delta) * P.scale, p1 * (__uint_as_float(dv[jj + 1]) - delta) * P.scale, P.fmt)
                           : 0u;
+            if constexpr (BIAS) {
+              gs[2 * e] = p0 * (__uint_as_float(dv[jj]) - delta);
+              gs[2 * e + 1] = p1 * (__uint_as_float(dv[jj + 1]) - delta);
+            }
+          }
+          if constexpr (BIAS) {
+            if (valid) {   // unscaled dS of this row into the row's own workspace slot (f32, unrounded)
+              float4* wp = reinterpret_cast<float4*>(wrow + c * 8);
+              float4 w0 = wp[0], w1 = wp[1];
+              w0.x += gs[0]; w0.y += gs[1]; w0.z += gs[2]; w0.w += gs[3];
+              w1.x += gs[4]; w1.y += gs[5]; w1.z += gs[6]; w1.w += gs[7];
+              wp[0] = w0; wp[1] = w1;
+            }
           }
           *reinterpret_cast<uint4*>(prow + sw128_offset(i, c)) = make_uint4(pw[0], pw[1], pw[2], pw[3]);
           *reinterpret_cast<uint4*>(drow + sw128_offset(i, c)) = make_uint4(dw[0], dw[1], dw[2], dw[3]);
@@ -693,24 +749,25 @@ swin_attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_
   if (warp == 9) { fence_after_sync(); tmem_dealloc(tmem_base, Cfg::TMEM_COLS); }
 }
 
-template <int HD>
-int launch_bwd(const void* qkv, const float* lse, const void* go, void* gqkv, long long T, int L, int C, int nh, const ShiftMask& M, int dtype,
-               cudaStream_t st) {
+template <int HD, bool BIAS>
+int launch_bwd(const void* qkv, const float* lse, const void* go, const float* bias, void* gqkv, float* dws, long long T, int L, int C, int nh,
+               const ShiftMask& M, int dtype, cudaStream_t st) {
   using Cfg = BCfg<HD>;
   const CUtensorMap* m = tensor_map_2d(qkv, (uint64_t)T, (uint64_t)3 * C, (uint64_t)3 * C, (uint32_t)L, 64, dtype);
   const CUtensorMap* mg = tensor_map_2d(go, (uint64_t)T, (uint64_t)C, (uint64_t)C, (uint32_t)L, 64, dtype);
   const CUtensorMap* mo = tensor_map_2d(gqkv, (uint64_t)T, (uint64_t)3 * C, (uint64_t)3 * C, (uint32_t)L, 64, dtype);
   if (!m || !mg || !mo) return B200_ERR_LAUNCH;
   AttnBwdParams P;
-  P.gqkv = gqkv; P.lse = lse; P.T = T; P.L = L; P.C = C; P.nh = nh; P.mask = M;
+  P.gqkv = gqkv; P.lse = lse; P.T = T; P.L = L; P.C = C; P.nh = nh; P.mask = M; P.bias = bias; P.dws = dws;
   P.n_items = (int)(T / L) * nh;
   P.n_pairs = (P.n_items + 1) / 2;
   P.fmt = dtype == B200_BF16 ? 1 : 0;
   P.scale = 1.f / sqrtf((float)HD);
   P.scale_log2 = 1.4426950408889634f * P.scale;
-  auto k = swin_attn_bwd_tc_kernel<HD>;
+  auto k = swin_attn_bwd_tc_kernel<HD, BIAS>;
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::TOTAL);
   int grid = P.n_pairs < sm_count() ? P.n_pairs : sm_count();
+  if (BIAS && grid > kRpbTcCtas) grid = kRpbTcCtas;   // the dS slots are sized for at most kRpbTcCtas CTAs
   k<<<grid, kThreads10, Cfg::TOTAL, st>>>(*m, *mg, *mo, P);
   return check_launch("swin_attn_bwd_tc");
 }
@@ -738,9 +795,9 @@ extern "C" B200_API int b200_swin_attn_fwd_tc(const void* qkv, void* o, float* l
   B200_REQUIRE(qkv && o, B200_ERR_SHAPE, "swin_attn_fwd_tc: null pointer");
   B200_REQUIRE((((uintptr_t)qkv | (uintptr_t)o) & 15) == 0, B200_ERR_ALIGN, "swin_attn_fwd_tc: 16-byte alignment required");
   cudaStream_t st = (cudaStream_t)stream;
-  if (C / nh == 64) return tc::launch_fwd<64>(qkv, o, lse, tokens, L, C, nh, M, dtype, st);
-  if (C / nh == 192) return tc::launch_fwd<192>(qkv, o, lse, tokens, L, C, nh, M, dtype, st);
-  return tc::launch_fwd<128>(qkv, o, lse, tokens, L, C, nh, M, dtype, st);
+  if (C / nh == 64) return tc::launch_fwd<64, false>(qkv, nullptr, o, lse, tokens, L, C, nh, M, dtype, st);
+  if (C / nh == 192) return tc::launch_fwd<192, false>(qkv, nullptr, o, lse, tokens, L, C, nh, M, dtype, st);
+  return tc::launch_fwd<128, false>(qkv, nullptr, o, lse, tokens, L, C, nh, M, dtype, st);
 }
 
 extern "C" B200_API int b200_swin_attn_bwd_tc(const void* qkv, const float* lse, const void* go, void* gqkv, int64_t tokens,
@@ -753,7 +810,53 @@ extern "C" B200_API int b200_swin_attn_bwd_tc(const void* qkv, const float* lse,
   B200_REQUIRE(qkv && lse && go && gqkv, B200_ERR_SHAPE, "swin_attn_bwd_tc: null pointer");
   B200_REQUIRE((((uintptr_t)qkv | (uintptr_t)go | (uintptr_t)gqkv) & 15) == 0, B200_ERR_ALIGN, "swin_attn_bwd_tc: 16-byte alignment required");
   cudaStream_t st = (cudaStream_t)stream;
-  if (C / nh == 64) return tc::launch_bwd<64>(qkv, lse, go, gqkv, tokens, L, C, nh, M, dtype, st);
-  if (C / nh == 192) return tc::launch_bwd<192>(qkv, lse, go, gqkv, tokens, L, C, nh, M, dtype, st);
-  return tc::launch_bwd<128>(qkv, lse, go, gqkv, tokens, L, C, nh, M, dtype, st);
+  if (C / nh == 64) return tc::launch_bwd<64, false>(qkv, lse, go, nullptr, gqkv, nullptr, tokens, L, C, nh, M, dtype, st);
+  if (C / nh == 192) return tc::launch_bwd<192, false>(qkv, lse, go, nullptr, gqkv, nullptr, tokens, L, C, nh, M, dtype, st);
+  return tc::launch_bwd<128, false>(qkv, lse, go, nullptr, gqkv, nullptr, tokens, L, C, nh, M, dtype, st);
+}
+
+extern "C" B200_API int b200_swin_attn_fwd_tc_rpb(const void* qkv, const float* bias, void* o, float* lse, int64_t tokens, int32_t L,
+                                                  int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift,
+                                                  int32_t dtype, void* stream) {
+  if (int rc = check_rpb(L, ws)) return rc;
+  if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
+  const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
+  B200_REQUIRE(b200_swin_attn_tc_supported(tokens, L, C, nh, dtype), B200_ERR_UNSUPPORTED,
+               "swin_attn_fwd_tc_rpb: unsupported problem (16-bit dtype, L<=64, head dim 64, 128 or 192)");
+  B200_REQUIRE(qkv && bias && o, B200_ERR_SHAPE, "swin_attn_fwd_tc_rpb: null pointer");
+  B200_REQUIRE((((uintptr_t)qkv | (uintptr_t)o | (uintptr_t)bias) & 15) == 0, B200_ERR_ALIGN, "swin_attn_fwd_tc_rpb: 16-byte alignment required");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (C / nh == 64) return tc::launch_fwd<64, true>(qkv, bias, o, lse, tokens, L, C, nh, M, dtype, st);
+  if (C / nh == 192) return tc::launch_fwd<192, true>(qkv, bias, o, lse, tokens, L, C, nh, M, dtype, st);
+  return tc::launch_fwd<128, true>(qkv, bias, o, lse, tokens, L, C, nh, M, dtype, st);
+}
+
+extern "C" B200_API int b200_swin_attn_bwd_tc_rpb(const void* qkv, const float* lse, const void* go, const float* bias, void* gqkv,
+                                                  float* gtable, int32_t table_rows, void* workspace, size_t workspace_bytes, int64_t tokens,
+                                                  int32_t L, int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift,
+                                                  int32_t dtype, void* stream) {
+  if (int rc = check_rpb(L, ws)) return rc;
+  if (int rc = check_shift(tokens, L, nWh, nWw, ws, shift)) return rc;
+  const ShiftMask M = make_shift_mask(nWh, nWw, ws, shift);
+  B200_REQUIRE(b200_swin_attn_tc_supported(tokens, L, C, nh, dtype), B200_ERR_UNSUPPORTED,
+               "swin_attn_bwd_tc_rpb: unsupported problem (16-bit dtype, L<=64, head dim 64, 128 or 192)");
+  B200_REQUIRE(table_rows == (2 * ws - 1) * (2 * ws - 1), B200_ERR_SHAPE, "swin_attn_bwd_tc_rpb: table has %d rows, ws %d needs %d",
+               table_rows, ws, (2 * ws - 1) * (2 * ws - 1));
+  B200_REQUIRE(qkv && lse && go && bias && gqkv && gtable && workspace, B200_ERR_SHAPE, "swin_attn_bwd_tc_rpb: null pointer");
+  B200_REQUIRE((((uintptr_t)qkv | (uintptr_t)go | (uintptr_t)gqkv | (uintptr_t)bias | (uintptr_t)workspace) & 15) == 0, B200_ERR_ALIGN,
+               "swin_attn_bwd_tc_rpb: 16-byte alignment required");
+  const long long pairs = (tokens / L * nh + 1) / 2;
+  const long long nslots = 4 * (pairs < kRpbTcCtas ? pairs : kRpbTcCtas);   // [CTA][warp group][item slot]
+  B200_REQUIRE(workspace_bytes >= rpb_workspace_bytes(nslots, nh), B200_ERR_WORKSPACE, "swin_attn_bwd_tc_rpb: workspace %zu < %zu bytes",
+               workspace_bytes, rpb_workspace_bytes(nslots, nh));
+  cudaStream_t st = (cudaStream_t)stream;
+  const cudaError_t e = cudaMemsetAsync(workspace, 0, (size_t)nslots * nh * 4096 * sizeof(float), st);
+  B200_REQUIRE(e == cudaSuccess, B200_ERR_LAUNCH, "swin_attn_bwd_tc_rpb: clearing the workspace failed: %s", cudaGetErrorString(e));
+  float* dws = (float*)workspace;
+  int rc;
+  if (C / nh == 64) rc = tc::launch_bwd<64, true>(qkv, lse, go, bias, gqkv, dws, tokens, L, C, nh, M, dtype, st);
+  else if (C / nh == 192) rc = tc::launch_bwd<192, true>(qkv, lse, go, bias, gqkv, dws, tokens, L, C, nh, M, dtype, st);
+  else rc = tc::launch_bwd<128, true>(qkv, lse, go, bias, gqkv, dws, tokens, L, C, nh, M, dtype, st);
+  if (rc) return rc;
+  return rpb_fold(dws, nslots, nh, ws, gtable, st);
 }

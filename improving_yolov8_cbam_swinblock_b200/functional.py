@@ -22,6 +22,12 @@ _lib.register("b200_swin_attn_bwd", C.c_int, [_VP] * 5 + [_I64] + [_I32] * 8 + [
 _lib.register("b200_swin_attn_tc_supported", C.c_int, [_I64] + [_I32] * 4)
 _lib.register("b200_swin_attn_fwd_tc", C.c_int, [_VP] * 3 + [_I64] + [_I32] * 8 + [_VP])
 _lib.register("b200_swin_attn_bwd_tc", C.c_int, [_VP] * 4 + [_I64] + [_I32] * 8 + [_VP])
+_lib.register("b200_swin_rpb_expand", C.c_int, [_VP, _I32, _VP, _I32, _I32, _VP])
+_lib.register("b200_swin_rpb_workspace_bytes", _SZ, [_I64, _I32, _I32, _I32])
+_lib.register("b200_swin_attn_fwd_rpb", C.c_int, [_VP] * 4 + [_I64] + [_I32] * 8 + [_VP])
+_lib.register("b200_swin_attn_bwd_rpb", C.c_int, [_VP] * 7 + [_I32, _VP, _SZ, _I64] + [_I32] * 8 + [_VP])
+_lib.register("b200_swin_attn_fwd_tc_rpb", C.c_int, [_VP] * 4 + [_I64] + [_I32] * 8 + [_VP])
+_lib.register("b200_swin_attn_bwd_tc_rpb", C.c_int, [_VP] * 6 + [_I32, _VP, _SZ, _I64] + [_I32] * 8 + [_VP])
 _lib.register("b200_swin_res_ln2", C.c_int, [_VP] * 8 + [_I64] + [_I32] * 2 + [_VP])
 _lib.register("b200_swin_gelu", C.c_int, [_VP] * 3 + [_I64] + [_I32] * 2 + [_VP])
 _lib.register("b200_swin_res_reverse", C.c_int, [_VP] * 3 + [_I32] * 7 + [_VP])
@@ -856,28 +862,58 @@ def _colsum(a: torch.Tensor) -> torch.Tensor:
 USE_TC_ATTENTION = True  # tests flip this to compare against the SIMT attention kernels
 
 
-def attn_forward(qkv, T, Lw, Cc, nh, grid=(0, 0, 0, 0)):
+def attn_forward(qkv, T, Lw, Cc, nh, grid=(0, 0, 0, 0), bias=None):
     """windowed MHSA on packed qkv[T,3C] -> (o[T,C], lse[T,nh]).  grid = (nWh, nWw, ws, shift): shifted-window mask
-    (extension; shift 0 = the reference's unmasked attention)."""
+    (extension; shift 0 = the reference's unmasked attention).  bias: dense relative-position bias [nh,64,64] f32 from
+    rpb_expand (SwinBlockRPB), added to the scores before the softmax; grid must then carry ws."""
     dev, code = qkv.device, dtype_code(qkv.dtype)
     o = torch.empty((T, Cc), dtype=qkv.dtype, device=dev)
     lse = torch.empty((T, nh), dtype=torch.float32, device=dev)
-    if USE_TC_ATTENTION and lib().b200_swin_attn_tc_supported(T, Lw, Cc, nh, code):
+    tc = USE_TC_ATTENTION and lib().b200_swin_attn_tc_supported(T, Lw, Cc, nh, code)
+    if bias is not None:
+        call("b200_swin_attn_fwd_tc_rpb" if tc else "b200_swin_attn_fwd_rpb", ptr(qkv), ptr(bias), ptr(o), ptr(lse), T, Lw, Cc, nh, *grid,
+             code, stream_ptr(dev))
+    elif tc:
         call("b200_swin_attn_fwd_tc", ptr(qkv), ptr(o), ptr(lse), T, Lw, Cc, nh, *grid, code, stream_ptr(dev))
     else:
         call("b200_swin_attn_fwd", ptr(qkv), ptr(o), ptr(lse), T, Lw, Cc, nh, *grid, code, stream_ptr(dev))
     return o, lse
 
 
-def attn_backward(qkv, o, lse, go, T, Lw, Cc, nh, grid=(0, 0, 0, 0)):
-    """gradient of attn_forward w.r.t. the packed qkv rows."""
+def attn_backward(qkv, o, lse, go, T, Lw, Cc, nh, grid=(0, 0, 0, 0), bias=None):
+    """gradient of attn_forward w.r.t. the packed qkv rows; with ``bias`` -> (gqkv, gtable [(2ws-1)^2, nh] f32), the
+    gradient of the relative-position bias table that ``bias`` was expanded from."""
     dev, code = qkv.device, dtype_code(qkv.dtype)
     gqkv = torch.empty_like(qkv)
-    if USE_TC_ATTENTION and lib().b200_swin_attn_tc_supported(T, Lw, Cc, nh, code):
+    tc = USE_TC_ATTENTION and lib().b200_swin_attn_tc_supported(T, Lw, Cc, nh, code)
+    if bias is not None:
+        ws = grid[2]
+        rows = (2 * ws - 1) ** 2
+        gtable = torch.empty((rows, nh), dtype=torch.float32, device=dev)
+        nbytes = lib().b200_swin_rpb_workspace_bytes(T, Lw, nh, int(tc))
+        wsb = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        if tc:
+            call("b200_swin_attn_bwd_tc_rpb", ptr(qkv), ptr(lse), ptr(go), ptr(bias), ptr(gqkv), ptr(gtable), rows, ptr(wsb), nbytes, T, Lw,
+                 Cc, nh, *grid, code, stream_ptr(dev))
+        else:
+            call("b200_swin_attn_bwd_rpb", ptr(qkv), ptr(o), ptr(lse), ptr(go), ptr(bias), ptr(gqkv), ptr(gtable), rows, ptr(wsb), nbytes,
+                 T, Lw, Cc, nh, *grid, code, stream_ptr(dev))
+        return gqkv, gtable
+    if tc:
         call("b200_swin_attn_bwd_tc", ptr(qkv), ptr(lse), ptr(go), ptr(gqkv), T, Lw, Cc, nh, *grid, code, stream_ptr(dev))
     else:
         call("b200_swin_attn_bwd", ptr(qkv), ptr(o), ptr(lse), ptr(go), ptr(gqkv), T, Lw, Cc, nh, *grid, code, stream_ptr(dev))
     return gqkv
+
+
+def rpb_expand(table: torch.Tensor, ws: int) -> torch.Tensor:
+    """relative_position_bias_table [(2ws-1)^2, nh] (any float dtype) -> dense f32 bias [nh, 64, 64] (rows / columns >= ws*ws
+    zero), the form the attention kernels read."""
+    t = _f32(table)
+    rows, nh = t.shape
+    bias = torch.empty((nh, 64, 64), dtype=torch.float32, device=t.device)
+    call("b200_swin_rpb_expand", ptr(t), rows, ptr(bias), ws, nh, stream_ptr(t.device))
+    return bias
 
 
 USE_FUSED_ATTN = True  # tests flip this to compare the fused tcgen05 attention half with the unfused stage-by-stage path
@@ -966,7 +1002,7 @@ class SwinBlockFn(torch.autograd.Function):
             return SwinBlockFn._backward(ctx, gout)
 
     @staticmethod
-    def _forward(ctx, x, g1, b1, win, bin_, wo, bo, g2, b2, w1, bb1, w2, bb2, num_heads, ws, shift):
+    def _forward(ctx, x, g1, b1, win, bin_, wo, bo, g2, b2, w1, bb1, w2, bb2, num_heads, ws, shift, rpb=None):
         from . import gemm
 
         x = _nhwc(x)
@@ -982,7 +1018,10 @@ class SwinBlockFn(torch.autograd.Function):
         need_grad = any(ctx.needs_input_grad)
         with torch.cuda.device(dev):
             grid = (-(-H // ws), -(-W // ws), ws, shift)
-            fused_attn = fused_attn_supported(B, Cc, H, W, num_heads, ws, shift, dt) and fused_mlp_supported(B * H * W, Cc, dt)
+            # the fused attention half takes no relative-position bias: with a table the attention half runs stage by stage
+            fused_attn = (rpb is None and fused_attn_supported(B, Cc, H, W, num_heads, ws, shift, dt)
+                          and fused_mlp_supported(B * H * W, Cc, dt))
+            bias = rpb_expand(rpb, ws) if rpb is not None else None
             if fused_attn:
                 # attention half in one tcgen05 kernel: x -> y1 in pixel order (+ the backward's by-products when training)
                 if need_grad:
@@ -997,7 +1036,7 @@ class SwinBlockFn(torch.autograd.Function):
                 call("b200_swin_ln1_partition", ptr(x), ptr(g1f), ptr(b1f), ptr(n1), ptr(mean1), ptr(rstd1), B, Cc, H, W, ws,
                                                 shift, code, st)
                 qkv = gemm.linear(n1, win, bin_)
-                o, lse = attn_forward(qkv, T, Lw, Cc, num_heads, grid)
+                o, lse = attn_forward(qkv, T, Lw, Cc, num_heads, grid, bias)
                 y1 = gemm.linear_res(o, wo, bo, n1)  # post-norm residual fused into the out_proj epilogue
             fused = fused_mlp_supported(B * H * W, Cc, dt)
             if fused:
@@ -1022,8 +1061,9 @@ class SwinBlockFn(torch.autograd.Function):
                 call("b200_swin_res_reverse", ptr(y1), ptr(m), ptr(out), B, Cc, H, W, ws, shift, code, st)
                 ctx.save_for_backward(x, g1f, g2f, win, wo, w1, w2, n1, mean1, rstd1, qkv, o, lse, y1, u, mean2, rstd2, hpre, h)
         ctx.fused_mlp = fused
+        ctx.bias = bias
         ctx.cfg = (B, Cc, H, W, ws, num_heads, T, shift)
-        ctx.pdtypes = tuple(p.dtype for p in (g1, b1, win, bin_, wo, bo, g2, b2, w1, bb1, w2, bb2))
+        ctx.pdtypes = tuple(p.dtype for p in (g1, b1, win, bin_, wo, bo, g2, b2, w1, bb1, w2, bb2) + ((rpb,) if rpb is not None else ()))
         return out
 
     @staticmethod
@@ -1078,7 +1118,11 @@ class SwinBlockFn(torch.autograd.Function):
             # attention
             gwo, gbo = gemm.matmul_tn(gy1, o)     # [C, C], [C]
             go = gemm.matmul_nn(gy1, wo)          # [T, C]
-            gqkv = attn_backward(qkv, o, lse, go.contiguous(), T, Lw, Cc, nh, grid)
+            gtable = None
+            if ctx.bias is None:
+                gqkv = attn_backward(qkv, o, lse, go.contiguous(), T, Lw, Cc, nh, grid)
+            else:
+                gqkv, gtable = attn_backward(qkv, o, lse, go.contiguous(), T, Lw, Cc, nh, grid, ctx.bias)
             del go
             gwin, gbin = gemm.matmul_tn(gqkv, n1)  # [3C, C], [3C]
             gn1 = gemm.matmul_nn(gqkv, win, add=gy1)  # [T, C] = gy1 + gqkv Win
@@ -1089,15 +1133,17 @@ class SwinBlockFn(torch.autograd.Function):
             gbt1 = torch.empty(Cc, dtype=torch.float32, device=dev)
             call("b200_swin_ln_bwd", ptr(gn1), ptr(x), None, ptr(g1f), ptr(mean1), ptr(rstd1), ptr(gx), ptr(gg1),
                                      ptr(gbt1), ptr(wsb), nbytes, B, Cc, H, W, ws, shift, code, 1, st)
-        grads = [gg1, gbt1, gwin, gbin, gwo, gbo, gg2, gbt2, gw1, gb1, gw2, gb2]
+        grads = [gg1, gbt1, gwin, gbin, gwo, gbo, gg2, gbt2, gw1, gb1, gw2, gb2] + ([gtable] if gtable is not None else [])
         grads = [g.to(d) for g, d in zip(grads, ctx.pdtypes)]
-        return (gx, *grads, None, None, None)
+        return (gx, *grads[:12], None, None, None, grads[12] if gtable is not None else None)
 
 
-def swin_block(x, p: dict, num_heads: int, ws: int, shift: int = 0):
+def swin_block(x, p: dict, num_heads: int, ws: int, shift: int = 0, rpb: torch.Tensor | None = None):
     """p: parameters keyed like the reference state_dict (norm1.weight, attn.in_proj_weight, ...).
     shift > 0: shifted-window extension (cyclic shift folded into the token addressing, seam mask applied in registers
     before the softmax); 0 = the reference block (swin_block.py has no shift, SURVEY D1).
+    rpb: relative_position_bias_table [(2ws-1)^2, num_heads] of SwinBlockRPB (extension, Swin's learned bias; ws <= 8), or
+    None (the reference block).  With a table the attention half runs stage by stage (the fused attention half takes no bias).
 
     Compute dtype = the autocast dtype when autocast is on (the reference runs its GEMMs there; trainer.py:383),
     else x.dtype."""
@@ -1106,4 +1152,4 @@ def swin_block(x, p: dict, num_heads: int, ws: int, shift: int = 0):
     return SwinBlockFn.apply(
         x, p["norm1.weight"], p["norm1.bias"], p["attn.in_proj_weight"], p["attn.in_proj_bias"],
         p["attn.out_proj.weight"], p["attn.out_proj.bias"], p["norm2.weight"], p["norm2.bias"],
-        p["mlp.0.weight"], p["mlp.0.bias"], p["mlp.2.weight"], p["mlp.2.bias"], num_heads, ws, int(shift))
+        p["mlp.0.weight"], p["mlp.0.bias"], p["mlp.2.weight"], p["mlp.2.bias"], num_heads, ws, int(shift), rpb)

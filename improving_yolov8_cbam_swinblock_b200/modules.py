@@ -132,17 +132,47 @@ class SwinBlock(nn.Module):
         if x.shape[1] != self.dim:
             raise RuntimeError(f"Given normalized_shape=[{self.dim}], expected input with {self.dim} channels, "
                                f"got {tuple(x.shape)}")
-        p = {
-            "norm1.weight": self.norm1.weight, "norm1.bias": self.norm1.bias,
-            "attn.in_proj_weight": self.attn.in_proj_weight, "attn.in_proj_bias": self.attn.in_proj_bias,
-            "attn.out_proj.weight": self.attn.out_proj.weight, "attn.out_proj.bias": self.attn.out_proj.bias,
-            "norm2.weight": self.norm2.weight, "norm2.bias": self.norm2.bias,
-            "mlp.0.weight": self.mlp[0].weight, "mlp.0.bias": self.mlp[0].bias,
-            "mlp.2.weight": self.mlp[2].weight, "mlp.2.bias": self.mlp[2].bias,
-        }
         # num_heads / shift come from state the reference class also has: a module pickled by the reference and unpickled
         # after plugin.install() (tasks.py:1222) never ran this __init__, so it has no `num_heads` / `shift_size` attribute
-        return Fb.swin_block(x, p, self.attn.num_heads, self.window_size, getattr(self, "shift_size", 0))
+        return Fb.swin_block(x, _swin_params(self), self.attn.num_heads, self.window_size, getattr(self, "shift_size", 0))
+
+
+def _swin_params(m: SwinBlock) -> dict:
+    """A SwinBlock's parameters keyed like the reference state_dict (what functional.swin_block takes)."""
+    return {
+        "norm1.weight": m.norm1.weight, "norm1.bias": m.norm1.bias,
+        "attn.in_proj_weight": m.attn.in_proj_weight, "attn.in_proj_bias": m.attn.in_proj_bias,
+        "attn.out_proj.weight": m.attn.out_proj.weight, "attn.out_proj.bias": m.attn.out_proj.bias,
+        "norm2.weight": m.norm2.weight, "norm2.bias": m.norm2.bias,
+        "mlp.0.weight": m.mlp[0].weight, "mlp.0.bias": m.mlp[0].bias,
+        "mlp.2.weight": m.mlp[2].weight, "mlp.2.bias": m.mlp[2].bias,
+    }
+
+
+class SwinBlockRPB(SwinBlock):
+    """SwinBlock with Swin's learned relative-position bias (Liu et al. 2021, eq. 4) added to the attention scores:
+    S[h,i,j] = q_i.k_j / sqrt(hd) + table[idx(i,j), h], idx = Swin's relative_position_index of the two tokens' positions in
+    their window (computed, not stored).  EXTENSION, opt-in: the reference block has no bias (SURVEY D1).
+
+    One parameter beyond SwinBlock's, ``relative_position_bias_table`` [(2ws-1)^2, num_heads] f32, trunc_normal(std=0.02)
+    as in Swin; its name contains "bias", so the optimizer grouping (trainer.py:818-827) puts it in the no-decay group, as
+    Swin does.  A SwinBlock state_dict loads with strict=False (only the table is missing).  Windows up to 8x8."""
+
+    def __init__(self, dim, num_heads=2, window_size=7, shift_size=0):
+        if not 1 <= window_size <= 8:
+            raise ValueError(f"SwinBlockRPB supports window_size 1..8, got {window_size}")
+        super().__init__(dim, num_heads, window_size, shift_size)
+        self.relative_position_bias_table = nn.Parameter(torch.zeros((2 * window_size - 1) ** 2, num_heads))
+        nn.init.trunc_normal_(self.relative_position_bias_table, std=0.02)
+
+    def forward(self, x):
+        if not x.is_cuda:
+            return _shape_probe(x, "SwinBlockRPB")
+        if x.shape[1] != self.dim:
+            raise RuntimeError(f"Given normalized_shape=[{self.dim}], expected input with {self.dim} channels, "
+                               f"got {tuple(x.shape)}")
+        return Fb.swin_block(x, _swin_params(self), self.attn.num_heads, self.window_size, getattr(self, "shift_size", 0),
+                             self.relative_position_bias_table)
 
 
 FUSE_CONV_EPILOGUE = [True]  # process-wide switch (tests / A-B timing); False = the caller's stock BatchNorm2d + SiLU

@@ -21,12 +21,15 @@ from . import modules as _m
 _TARGETS = ("ultralytics.nn.tasks", "ultralytics.nn.modules", "ultralytics.nn.modules.cbam",
             "ultralytics.nn.modules.swin_block", "ultralytics.nn.modules.block")
 _saved: dict = {}
+_added: list = []   # (module, name) that install() created rather than rebound
+_NEW_TARGETS = ("ultralytics.nn.tasks", "ultralytics.nn.modules")
 _saved_methods: dict = {}
 
 CBAM = _m.CBAM
 ChannelAttentionMap = _m.ChannelAttention
 SpatialAttentionMap = _m.SpatialAttention
 SwinBlock = _m.SwinBlock
+SwinBlockRPB = _m.SwinBlockRPB   # extension: no such name in the reference, so install() adds it where parse_model looks
 SPPF = None  # created by install() against ultralytics' Conv
 Conv = None  # ultralytics' Conv with the fused BN+SiLU epilogue (SURVEY 8(f)-1), created by install()
 _CONV_TARGETS = ("ultralytics.nn.tasks", "ultralytics.nn.modules", "ultralytics.nn.modules.conv",
@@ -59,7 +62,9 @@ _SEAM_PATCHES = (("ultralytics.nn.modules.block", "C2f", "forward", _c2f_forward
 
 
 def install(conv_epilogue: bool = False, seams: bool = False):
-    """Rebind CBAM / SwinBlock / SPPF in the reference's namespaces.  Returns the {name: class} table.
+    """Rebind CBAM / SwinBlock / SPPF in the reference's namespaces and add SwinBlockRPB to ``ultralytics.nn.tasks`` /
+    ``ultralytics.nn.modules`` (so a yaml row ``[-1, 1, SwinBlockRPB, [128]]`` parses like SwinBlock).  Returns the
+    {name: class} table.
 
     SPPF's own cv1/cv2 always use the fused BN+SiLU epilogue; ``conv_epilogue=True`` additionally rebinds ``Conv``
     itself (a subclass of the reference's, same state_dict / ``fuse()`` behaviour) so every Conv caller gets it.
@@ -71,7 +76,7 @@ def install(conv_epilogue: bool = False, seams: bool = False):
         Conv = _m.make_conv(_saved.get(("ultralytics.nn.modules.conv", "Conv"), conv_mod.Conv), module=__name__)
     if SPPF is None:
         SPPF = _m.make_sppf(Conv, module=__name__)
-    table = {"CBAM": CBAM, "SwinBlock": SwinBlock, "SPPF": SPPF}
+    table = {"CBAM": CBAM, "SwinBlock": SwinBlock, "SPPF": SPPF, "SwinBlockRPB": SwinBlockRPB}
     if conv_epilogue:
         for modname in _CONV_TARGETS:
             mod = importlib.import_module(modname)
@@ -86,8 +91,12 @@ def install(conv_epilogue: bool = False, seams: bool = False):
     for modname in _TARGETS:
         mod = importlib.import_module(modname)
         for name, cls in table.items():
-            if hasattr(mod, name):
+            if hasattr(mod, name) and (modname, name) not in _added:
                 _saved.setdefault((modname, name), getattr(mod, name))
+                setattr(mod, name, cls)
+            elif modname in _NEW_TARGETS and name == "SwinBlockRPB":
+                if (modname, name) not in _added:
+                    _added.append((modname, name))
                 setattr(mod, name, cls)
     # cbam.py's own ChannelAttention / SpatialAttention (maps only).  NOTE: ultralytics.nn.modules exports the
     # *stock* conv.py classes under these names (modules/__init__.py:66,78; SURVEY D5) -- those are left alone.
@@ -102,6 +111,11 @@ def uninstall():
     for (modname, name), cls in list(_saved.items()):
         setattr(importlib.import_module(modname), name, cls)
     _saved.clear()
+    for modname, name in _added:
+        mod = importlib.import_module(modname)
+        if hasattr(mod, name):
+            delattr(mod, name)
+    _added.clear()
     for (modname, clsname, attr), fn in list(_saved_methods.items()):
         setattr(getattr(importlib.import_module(modname), clsname), attr, fn)
     _saved_methods.clear()

@@ -215,6 +215,36 @@ B200_API int b200_swin_attn_bwd_tc(const void* qkv, const float* lse, const void
                                    int32_t shift, int32_t dtype, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------
+ * Learned relative-position bias of window attention (SwinBlockRPB; EXTENSION: the reference block has none, SURVEY D1).
+ * Liu et al. 2021, "Swin Transformer: Hierarchical Vision Transformer using Shifted Windows", eq. 4:
+ *   S[h,i,j] = (q_i . k_j) * hd^-0.5 + table[idx(i,j), h]   (+ the shift mask when shift > 0)
+ *   idx(i,j) = (y_i - y_j + ws - 1) * (2ws - 1) + (x_i - x_j + ws - 1),  (y, x) = row / column of a token in its window
+ * table [(2ws-1)^2, nh] f32 (table_rows = (2ws-1)^2), 1 <= ws <= 8, L = ws*ws.  Padded and shifted windows use the same
+ * index by window position, as in Swin.  lse is that of the biased scores.
+ *   b200_swin_rpb_expand : table -> dense bias [nh][64][64] f32, rows / columns >= L zero (what the attention entries read)
+ *   *_fwd_rpb / *_fwd_tc_rpb : b200_swin_attn_fwd / _fwd_tc with the dense bias added to the scores before the softmax
+ *   *_bwd_rpb / *_bwd_tc_rpb : b200_swin_attn_bwd / _bwd_tc plus gtable [(2ws-1)^2, nh] f32 = dL/dtable, OVERWRITTEN and
+ *       run-to-run bit-identical (per-slot dS in `workspace`, folded in a fixed order; no atomics).  workspace:
+ *       b200_swin_rpb_workspace_bytes(tokens, L, nh, tc) bytes, tc = 1 for the _tc entry, 0 for the SIMT one.
+ * ------------------------------------------------------------------------------------------------------ */
+B200_API int b200_swin_rpb_expand(const float* table, int32_t table_rows, float* bias, int32_t ws, int32_t nh, void* stream);
+B200_API size_t b200_swin_rpb_workspace_bytes(int64_t tokens, int32_t L, int32_t nh, int32_t tc);
+B200_API int b200_swin_attn_fwd_rpb(const void* qkv, const float* bias, void* o, float* lse, int64_t tokens, int32_t L,
+                                    int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift, int32_t dtype,
+                                    void* stream);
+B200_API int b200_swin_attn_bwd_rpb(const void* qkv, const void* o, const float* lse, const void* go, const float* bias,
+                                    void* gqkv, float* gtable, int32_t table_rows, void* workspace, size_t workspace_bytes,
+                                    int64_t tokens, int32_t L, int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws,
+                                    int32_t shift, int32_t dtype, void* stream);
+B200_API int b200_swin_attn_fwd_tc_rpb(const void* qkv, const float* bias, void* o, float* lse, int64_t tokens, int32_t L,
+                                       int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift, int32_t dtype,
+                                       void* stream);
+B200_API int b200_swin_attn_bwd_tc_rpb(const void* qkv, const float* lse, const void* go, const float* bias, void* gqkv,
+                                       float* gtable, int32_t table_rows, void* workspace, size_t workspace_bytes, int64_t tokens,
+                                       int32_t L, int32_t C, int32_t nh, int32_t nWh, int32_t nWw, int32_t ws, int32_t shift,
+                                       int32_t dtype, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------
  * Conv epilogue -- replaces `self.act(self.bn(y))` of Conv.forward (ultralytics/nn/modules/conv.py:65-79:
  * BatchNorm2d then SiLU) on the conv output y, for SPPF's cv1/cv2 (block.py:218-219; SURVEY section 8(f)-1) and the
  * other Conv callers either side of the path.  x/z/gz/gx: NHWC viewed as [rows = B*H*W, C] in the activation dtype;
